@@ -2,6 +2,7 @@
 """Headline benchmark: cuda_allreduce_ring_chunked, float32, on N B200s of one node.
 
     python bench.py --gpus 1 --steps 20 --warmup 5
+    python bench.py --gpus 1 --steps 20 --warmup 5 --dump-outputs DIR   # + the last step's buffers as DIR/*.npy
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29500 bench.py --gpus 8 --steps 20 --warmup 5
     ... bench.py --impl reference ...   # unmodified pytorch/gloo benchmark_cuda from baseline/_ref
@@ -43,6 +44,8 @@ METRIC = ("cuda_allreduce_ring_chunked float32 aggregate bus bandwidth (GB/s sum
 PUBLISHED_BUSBW_GBS = 2.8  # BASELINE.md: 20 MB allreduce_ring_chunked, 4 machines, 40 GbE (derived busbw)
 HEADLINE_ELEMENTS = 100_000_000
 SWEEP = [1, 10, 100, 1_000, 10_000, 100_000, 1_000_000, 10_000_000]
+DUMP_BYTES = 32 << 20  # --dump-outputs budget over all ranks; larger outputs are sampled down to it
+DUMP_SEED = 0
 
 
 def env_int(name, dflt):
@@ -105,6 +108,26 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(out_dir, tensors, rank, world):
+    """Writes the buffers a step hands back to its caller as <out_dir>/rank<r>_buffer<i>.npy (float32).
+    A buffer larger than its share of DUMP_BYTES is cut into that many equal slices and reduced to
+    one value per slice, at a position drawn from DUMP_SEED: the same positions on every run, so two
+    builds compare element for element."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    per = DUMP_BYTES // 4 // (world * len(tensors))
+    for i, t in enumerate(tensors):
+        n = t.numel()
+        if n > per:
+            lo = np.arange(per, dtype=np.int64) * n // per
+            hi = np.append(lo[1:], n)
+            idx = np.random.default_rng(DUMP_SEED).integers(lo, hi)
+            t = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(out_dir, f"rank{rank}_buffer{i}.npy"), t.float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------
@@ -348,6 +371,8 @@ def run_ours(args):
     launches = cu.launch_count() - launches0
     total_ms = float(host_max([ev0.elapsed_time(ev1)])[0])
     ms_per_step = total_ms / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ts, rank, world)
     with torch.cuda.stream(stream):
         fill_inputs(ts)
         algo.run()
@@ -815,7 +840,14 @@ def main():
     ap.add_argument("--quick", action="store_true", help="headline + e2e + latency sweep only (skip BASELINE configs 3-5)")
     ap.add_argument("--no-verify-matrix", action="store_true", help="skip the multi-GPU correctness matrix before timing")
     ap.add_argument("--e2e-chunks", type=int, default=16, help="pieces of the host<->device pipeline in the e2e run")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the buffers of the last timed headline step to DIR/*.npy (float32, seeded sample "
+                         f"when they exceed {DUMP_BYTES >> 20} MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)
