@@ -149,16 +149,18 @@ CudaAllreduceCore::CudaAllreduceCore(std::shared_ptr<Context> ctx, std::vector<v
   }
   // Fold the extra local pointers inside the collective kernel when they live on the same
   // device as the first one (and, across ranks, every pointer is 16-byte aligned so that
-  // all ranks pick the same element -> CTA mapping).
+  // all ranks pick the same element -> CTA mapping). A single rank needs no alignment: its
+  // fused kernel takes unaligned pointers element by element and still rounds once.
   if (ptrs_.size() > 1 && ptrs_.size() - 1 <= static_cast<size_t>(kMaxLocal) && !envFlag("CUDA_NO_LOCAL_FUSION", false)) {
-    bool mine = true;
+    bool sameDevice = true, aligned = true;
     for (size_t i = 0; i < ptrs_.size(); i++) {
-      mine = mine && streams_[i].getDeviceID() == dev0 && reinterpret_cast<uintptr_t>(ptrs_[i]) % 16 == 0;
+      sameDevice = sameDevice && streams_[i].getDeviceID() == dev0;
+      aligned = aligned && reinterpret_cast<uintptr_t>(ptrs_[i]) % 16 == 0;
     }
     if (ctx_->size == 1) {
-      fuseLocal_ = mine;
+      fuseLocal_ = sameDevice;
     } else if (pc_ && !literal_) {
-      fuseLocal_ = pc_->agree(mine);
+      fuseLocal_ = pc_->agree(sameDevice && aligned);
     }
   }
   if (ctx_->size > 1 && !pc_) {

@@ -103,44 +103,6 @@ __device__ __forceinline__ void storeLocalGroup(T* out, const LocalPtrs& extra, 
 
 // ---- LL (flag in data) -------------------------------------------------------------------
 
-template <typename T>
-struct AccType {
-  using type = T;
-};
-template <>
-struct AccType<__half> {
-  using type = float;
-};
-template <>
-struct AccType<__nv_bfloat16> {
-  using type = float;
-};
-
-template <typename T>
-__device__ __forceinline__ typename AccType<T>::type toAcc(T x) {
-  return x;
-}
-template <>
-__device__ __forceinline__ float toAcc<__half>(__half x) {
-  return __half2float(x);
-}
-template <>
-__device__ __forceinline__ float toAcc<__nv_bfloat16>(__nv_bfloat16 x) {
-  return __bfloat162float(x);
-}
-template <typename TO, typename A>
-__device__ __forceinline__ TO fromAcc(A x) {
-  return static_cast<TO>(x);
-}
-template <>
-__device__ __forceinline__ __half fromAcc<__half, float>(float x) {
-  return __float2half_rn(x);
-}
-template <>
-__device__ __forceinline__ __nv_bfloat16 fromAcc<__nv_bfloat16, float>(float x) {
-  return __float2bfloat16_rn(x);
-}
-
 // `ll.p[r]` is the LL region of rank r's pool: [parity][source rank][line]. A launch uses
 // parity = seq & 1; two halves suffice because a rank can run at most one launch ahead of
 // its slowest peer (it needs that peer's lines of launch s+1 to finish launch s+1).
@@ -180,16 +142,37 @@ llAllreduceKernel(CommArgs a, const T* in, TO* out, size_t count, DevOp op, floa
         if (i0 + k < count) t[k] = in[i0 + k];
       }
     }
-    if (extra.n > 0) {
+    if constexpr (std::is_same<A, T>::value) {
+      if (extra.n > 0) {
+#pragma unroll
+        for (int e = 0; e < kMaxLocal; e++) {
+          if (e < extra.n) {
+            const T* x = static_cast<const T*>(extra.p[e]);
+#pragma unroll
+            for (int k = 0; k < K; k++) {
+              if (i0 + k < count) t[k] = applyOp<T>(t[k], x[i0 + k], op);
+            }
+          }
+        }
+      }
+    } else if (extra.n > 0) {
+      // the local fold is stored in T (peers read it): accumulate in A, round once
+      A f[K];
+#pragma unroll
+      for (int k = 0; k < K; k++) f[k] = toAcc<T>(t[k]);
 #pragma unroll
       for (int e = 0; e < kMaxLocal; e++) {
         if (e < extra.n) {
           const T* x = static_cast<const T*>(extra.p[e]);
 #pragma unroll
           for (int k = 0; k < K; k++) {
-            if (i0 + k < count) t[k] = PackTraits<T>::combineOne(t[k], x[i0 + k], op);
+            if (i0 + k < count) f[k] = applyOp<A>(f[k], toAcc<T>(x[i0 + k]), op);
           }
         }
+      }
+#pragma unroll
+      for (int k = 0; k < K; k++) {
+        if (i0 + k < count) t[k] = fromAcc<T, A>(f[k]);
       }
     }
     // push to every peer: posted NVLink stores, no round trip
@@ -449,9 +432,10 @@ __device__ __forceinline__ void foldLocalShares(char* mine, const LocalPtrs& ext
     size_t tb, te;
     shareOf(count - tailStart, P, r, tb, te);
     for (size_t i = tailStart + tb + tid; i < tailStart + te; i += nthreads) {
-      T acc = reinterpret_cast<T*>(mine)[i];
-      for (int k = 0; k < extra.n; k++) acc = PT::combineOne(acc, static_cast<const T*>(extra.p[k])[i], op);
-      reinterpret_cast<T*>(mine)[i] = acc;
+      using A = typename AccType<T>::type;
+      A acc = toAcc<T>(reinterpret_cast<T*>(mine)[i]);
+      for (int k = 0; k < extra.n; k++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(extra.p[k])[i]), op);
+      reinterpret_cast<T*>(mine)[i] = fromAcc<T, A>(acc);
     }
   }
 }
@@ -552,10 +536,12 @@ twoShotAllreduceKernel(CommArgs a, PeerPtrs bufs, size_t count, DevOp op, float 
     size_t tb, te;
     shareOf(count - tailStart, P, a.rank, tb, te);
     for (size_t i = tailStart + tb + tid; i < tailStart + te; i += nthreads) {
-      T acc = static_cast<const T*>(bufs.p[0])[i];
-      for (int r = 1; r < P; r++) acc = PT::combineOne(acc, static_cast<const T*>(bufs.p[r])[i], op);
-      if (scale != 1.0f) acc = PT::scaleOne(acc, scale);
-      for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = acc;
+      using A = typename AccType<T>::type;
+      A acc = toAcc<T>(static_cast<const T*>(bufs.p[0])[i]);
+      for (int r = 1; r < P; r++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(bufs.p[r])[i]), op);
+      if (scale != 1.0f) acc = scaleAcc(acc, scale);
+      const T res = fromAcc<T, A>(acc);
+      for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = res;
     }
   }
 
@@ -616,10 +602,12 @@ nvlsAllreduceKernel(CommArgs a, char* mcBase, PeerPtrs bufs, size_t count, float
     size_t tb, te;
     shareOf(count - tailStart, P, a.rank, tb, te);
     for (size_t i = tailStart + tb + tid; i < tailStart + te; i += nthreads) {
-      T acc = static_cast<const T*>(bufs.p[0])[i];
-      for (int r = 1; r < P; r++) acc = PT::combineOne(acc, static_cast<const T*>(bufs.p[r])[i], DevOp::SUM);
-      if (scale != 1.0f) acc = PT::scaleOne(acc, scale);
-      for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = acc;
+      using A = typename AccType<T>::type;
+      A acc = toAcc<T>(static_cast<const T*>(bufs.p[0])[i]);
+      for (int r = 1; r < P; r++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(bufs.p[r])[i]), DevOp::SUM);
+      if (scale != 1.0f) acc = scaleAcc(acc, scale);
+      const T res = fromAcc<T, A>(acc);
+      for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = res;
     }
   }
   if (blockBarrier(a, e + 2) && extra.n > 0) fanOutLocalShares<T>(mine, extra, nvec, count, P, tid, nthreads);
@@ -708,10 +696,12 @@ hybridAllreduceKernel(CommArgs a, char* mcBase, PeerPtrs bufs, size_t count, flo
     size_t tb, te;
     shareOf(count - tailStart, P, a.rank, tb, te);
     for (size_t i = tailStart + tb + tid; i < tailStart + te; i += nthreads) {
-      T acc = static_cast<const T*>(bufs.p[0])[i];
-      for (int r = 1; r < P; r++) acc = PT::combineOne(acc, static_cast<const T*>(bufs.p[r])[i], DevOp::SUM);
-      if (scale != 1.0f) acc = PT::scaleOne(acc, scale);
-      for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = acc;
+      using A = typename AccType<T>::type;
+      A acc = toAcc<T>(static_cast<const T*>(bufs.p[0])[i]);
+      for (int r = 1; r < P; r++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(bufs.p[r])[i]), DevOp::SUM);
+      if (scale != 1.0f) acc = scaleAcc(acc, scale);
+      const T res = fromAcc<T, A>(acc);
+      for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = res;
     }
   }
   blockBarrier(a, e + 2);

@@ -620,10 +620,11 @@ reducePullKernel(CommArgs a, PeerPtrs ins, char* mcIn, T* __restrict__ out, EArg
     }
   }
   for (size_t i = nvec * PT::kElems + tid; i < len; i += nthreads) {
-    T acc = static_cast<const T*>(ins.p[0])[off + i];
-    for (int r = 1; r < P; r++) acc = PT::combineOne(acc, static_cast<const T*>(ins.p[r])[off + i], op);
-    if (scale != 1.0f) acc = PT::scaleOne(acc, scale);
-    out[i] = acc;
+    using A = typename AccType<T>::type;
+    A acc = toAcc<T>(static_cast<const T*>(ins.p[0])[off + i]);
+    for (int r = 1; r < P; r++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(ins.p[r])[off + i]), op);
+    if (scale != 1.0f) acc = scaleAcc(acc, scale);
+    out[i] = fromAcc<T, A>(acc);
   }
   blockBarrier(a, e + 2);
   retire(a, 2, 0);

@@ -254,6 +254,8 @@ struct PackTraits {
     return p;
   }
   __device__ static T one(const T* p) { return *p; }
+  // combineOne / scaleOne round to T after every step. Only the literal schedules use them:
+  // they store each step's partial in T by design. Fused kernels go through AccType below.
   __device__ static T combineOne(T a, T b, DevOp op) { return applyOp<T>(a, b, op); }
   // Epilogue: multiply the reduced value (floating types only; the host rejects a scale
   // on integer buffers).
@@ -353,6 +355,54 @@ struct PackTraits<__nv_bfloat16> {
     return __float2bfloat16_rn(__bfloat162float(a) * s);
   }
 };
+
+// ---- one element at a time ---------------------------------------------------------------
+// The scalar paths (sub-pack tails, unaligned buffers, uneven shares) follow the same rule as
+// the packs: widen to AccType<T>, reduce and scale there, round once with fromAcc. AccType is
+// T itself for every type but the 16-bit floats, so integer / f32 / f64 arithmetic is plain T.
+template <typename T>
+struct AccType {
+  using type = T;
+};
+template <>
+struct AccType<__half> {
+  using type = float;
+};
+template <>
+struct AccType<__nv_bfloat16> {
+  using type = float;
+};
+
+template <typename T>
+__device__ __forceinline__ typename AccType<T>::type toAcc(T x) {
+  return x;
+}
+template <>
+__device__ __forceinline__ float toAcc<__half>(__half x) {
+  return __half2float(x);
+}
+template <>
+__device__ __forceinline__ float toAcc<__nv_bfloat16>(__nv_bfloat16 x) {
+  return __bfloat162float(x);
+}
+template <typename TO, typename A>
+__device__ __forceinline__ TO fromAcc(A x) {
+  return static_cast<TO>(x);
+}
+template <>
+__device__ __forceinline__ __half fromAcc<__half, float>(float x) {
+  return __float2half_rn(x);
+}
+template <>
+__device__ __forceinline__ __nv_bfloat16 fromAcc<__nv_bfloat16, float>(float x) {
+  return __float2bfloat16_rn(x);
+}
+// Epilogue on an accumulator (floating types only; the host rejects a scale on integers).
+template <typename A>
+__device__ __forceinline__ A scaleAcc(A x, float s) {
+  if constexpr (std::is_floating_point<A>::value) return static_cast<A>(x * s);
+  return x;
+}
 
 // ---- mixed-precision items (cast epilogue) --------------------------------------------
 // Eight consecutive elements of T as fp32 lanes: 2 x 16 B for float, 1 x 16 B for the

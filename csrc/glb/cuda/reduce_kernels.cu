@@ -47,9 +47,10 @@ localReduceManyKernel(T* __restrict__ dst, SrcPtrs srcs, int nsrc, size_t count,
     st128(reinterpret_cast<char*>(dst) + v * 16, PT::narrow(acc));
   }
   for (size_t i = nvec * PT::kElems + tid; i < count; i += nthreads) {
-    T acc = static_cast<const T*>(srcs.p[0])[i];
-    for (int s = 1; s < nsrc; s++) acc = PT::combineOne(acc, static_cast<const T*>(srcs.p[s])[i], op);
-    dst[i] = acc;
+    using A = typename AccType<T>::type;
+    A acc = toAcc<T>(static_cast<const T*>(srcs.p[0])[i]);
+    for (int s = 1; s < nsrc; s++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(srcs.p[s])[i]), op);
+    dst[i] = fromAcc<T, A>(acc);
   }
 }
 
@@ -90,10 +91,12 @@ localAllreduceManyKernel(DstPtrs bufs, int n, size_t count, DevOp op, float scal
     }
   }
   for (size_t i = nvec * PT::kElems + tid; i < count; i += nthreads) {
-    T acc = static_cast<const T*>(bufs.p[0])[i];
-    for (int s = 1; s < n; s++) acc = PT::combineOne(acc, static_cast<const T*>(bufs.p[s])[i], op);
-    if (scale != 1.0f) acc = PT::scaleOne(acc, scale);
-    for (int s = 0; s < n; s++) static_cast<T*>(bufs.p[s])[i] = acc;
+    using A = typename AccType<T>::type;
+    A acc = toAcc<T>(static_cast<const T*>(bufs.p[0])[i]);
+    for (int s = 1; s < n; s++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(bufs.p[s])[i]), op);
+    if (scale != 1.0f) acc = scaleAcc(acc, scale);
+    const T res = fromAcc<T, A>(acc);
+    for (int s = 0; s < n; s++) static_cast<T*>(bufs.p[s])[i] = res;
   }
 }
 
