@@ -32,6 +32,7 @@
 // There is no reference counterpart: the reference stages through pinned host
 // memory + TCP (cuda_allreduce_ring_chunked.cc:129-273) and reduces on the CPU.
 #include "glb/cuda/device_common.cuh"
+#include "glb/cuda/dispatch.cuh"
 #include "glb/cuda/kernels.h"
 
 namespace glb {
@@ -41,42 +42,6 @@ __global__ void barrierKernel(CommArgs a) {
   const uint32_t e = loadEpoch(a);
   blockBarrier(a, e + 1);
   retire(a, 1, 0);
-}
-
-// ---- element groups ------------------------------------------------------------------
-// The barrier pairs CTA b of one rank with CTA b of every peer, so which CTA touches which
-// element must not depend on anything rank-local (such as the alignment of a user pointer).
-// All staged kernels therefore own 16-byte *groups* of elements by index; a group is moved
-// with one 128-bit access when the pointer allows it and element by element otherwise.
-
-template <typename T>
-__device__ __forceinline__ Pack16 loadGroup(const T* base, size_t g, size_t count, bool aligned) {
-  constexpr int K = 16 / sizeof(T);
-  const size_t i0 = g * K;
-  if (aligned && i0 + K <= count) return ld128_stream(reinterpret_cast<const char*>(base) + g * 16);
-  Pack16 p;
-  p.w[0] = p.w[1] = p.w[2] = p.w[3] = 0u;
-  T* t = reinterpret_cast<T*>(&p);
-#pragma unroll
-  for (int k = 0; k < K; k++) {
-    if (i0 + k < count) t[k] = base[i0 + k];
-  }
-  return p;
-}
-
-template <typename T>
-__device__ __forceinline__ void storeGroup(T* base, size_t g, size_t count, bool aligned, const Pack16& p) {
-  constexpr int K = 16 / sizeof(T);
-  const size_t i0 = g * K;
-  if (aligned && i0 + K <= count) {
-    st128(reinterpret_cast<char*>(base) + g * 16, p);
-    return;
-  }
-  const T* t = reinterpret_cast<const T*>(&p);
-#pragma unroll
-  for (int k = 0; k < K; k++) {
-    if (i0 + k < count) base[i0 + k] = t[k];
-  }
 }
 
 // Group g of the local contribution: the first pointer, plus the extra local pointers
@@ -97,8 +62,8 @@ __device__ __forceinline__ Pack16 loadLocalGroup(const T* in, const LocalPtrs& e
 template <typename T>
 __device__ __forceinline__ void storeLocalGroup(T* out, const LocalPtrs& extra, size_t g, size_t count, bool aligned,
                                                 const Pack16& p) {
-  storeGroup(out, g, count, aligned, p);
-  for (int k = 0; k < extra.n; k++) storeGroup(static_cast<T*>(extra.p[k]), g, count, aligned, p);
+  storeGroup<false>(out, g, count, aligned, p);
+  for (int k = 0; k < extra.n; k++) storeGroup<false>(static_cast<T*>(extra.p[k]), g, count, aligned, p);
 }
 
 // ---- LL (flag in data) -------------------------------------------------------------------
@@ -406,13 +371,6 @@ oneShotAllreduceKernel(CommArgs a, const T* in, T* out, size_t count, DevOp op, 
 
 // ---- two-shot (fused reduce-scatter + allgather, in place) --------------------------
 
-// [begin, end) of rank r's share of n items.
-__device__ __forceinline__ void shareOf(size_t n, int parts, int r, size_t& begin, size_t& end) {
-  const size_t base = n / parts, rem = n % parts;
-  begin = r * base + (static_cast<size_t>(r) < rem ? r : rem);
-  end = begin + base + (static_cast<size_t>(r) < rem ? 1 : 0);
-}
-
 // Multi-pointer prologue: fold the extra local pointers into `mine`, share by share, with
 // the element -> (CTA, thread) mapping of the exchange phase (so the CTA that will read a
 // peer's element is the one that is barrier-paired with the CTA that folded it).
@@ -498,52 +456,10 @@ twoShotAllreduceKernel(CommArgs a, PeerPtrs bufs, size_t count, DevOp op, float 
 #pragma unroll
   for (int i = 0; i < kSlots; i++) peer[i] = i < P ? static_cast<char*>(bufs.p[(a.rank + i) % P]) : nullptr;
 
-  for (size_t v0 = vb + tid; v0 < ve; v0 += nthreads * UNROLL) {
-    Pack16 p[UNROLL][kSlots];
-#pragma unroll
-    for (int u = 0; u < UNROLL; u++) {
-      const size_t v = v0 + static_cast<size_t>(u) * nthreads;
-      if (v < ve) {
-#pragma unroll
-        for (int i = 0; i < kSlots; i++) {
-          if (i < P) p[u][i] = ld128_stream(peer[i] + v * 16);
-        }
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < UNROLL; u++) {
-      const size_t v = v0 + static_cast<size_t>(u) * nthreads;
-      if (v < ve) {
-        typename PT::AccPack acc = PT::widen(p[u][0]);
-#pragma unroll
-        for (int i = 1; i < kSlots; i++) {
-          if (i < P) PT::combine(acc, p[u][i], op);
-        }
-        if (scale != 1.0f) PT::scale(acc, scale);
-        const Pack16 res = PT::narrow(acc);
-#pragma unroll
-        for (int i = 0; i < kSlots; i++) {
-          if (i < P) st128_stream(peer[i] + v * 16, res);
-        }
-      }
-    }
-  }
-
-  // Scalar tail (count not a multiple of the pack width, or unaligned buffers):
-  // split across ranks the same way.
-  {
-    const size_t tailStart = nvec * PT::kElems;
-    size_t tb, te;
-    shareOf(count - tailStart, P, a.rank, tb, te);
-    for (size_t i = tailStart + tb + tid; i < tailStart + te; i += nthreads) {
-      using A = typename AccType<T>::type;
-      A acc = toAcc<T>(static_cast<const T*>(bufs.p[0])[i]);
-      for (int r = 1; r < P; r++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(bufs.p[r])[i]), op);
-      if (scale != 1.0f) acc = scaleAcc(acc, scale);
-      const T res = fromAcc<T, A>(acc);
-      for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = res;
-    }
-  }
+  peerAllreducePacks<T, kSlots, UNROLL>(peer, P, vb, ve, op, scale, tid, nthreads);
+  // Scalar tail (count not a multiple of the pack width, or unaligned buffers): split across
+  // ranks the same way.
+  allreduceTailInPlace<T>(bufs, P, a.rank, nvec * PT::kElems, count, op, scale, tid, nthreads);
 
   // All my stores have landed everywhere and nobody still reads my buffer.
   if (blockBarrier(a, e + 2) && extra.n > 0) fanOutLocalShares<T>(mine, extra, nvec, count, P, tid, nthreads);
@@ -551,14 +467,6 @@ twoShotAllreduceKernel(CommArgs a, PeerPtrs bufs, size_t count, DevOp op, float 
 }
 
 // ---- NVLS -----------------------------------------------------------------------------
-
-template <typename T>
-__device__ __forceinline__ Pack16 scalePack(const Pack16& p, float s) {
-  using PT = PackTraits<T>;
-  typename PT::AccPack acc = PT::widen(p);
-  PT::scale(acc, s);
-  return PT::narrow(acc);
-}
 
 template <typename T, int UNROLL>
 __global__ void __launch_bounds__(kThreads)
@@ -597,19 +505,7 @@ nvlsAllreduceKernel(CommArgs a, char* mcBase, PeerPtrs bufs, size_t count, float
     }
   }
   // Sub-pack tail through plain peer pointers, split like the two-shot tail.
-  {
-    const size_t tailStart = nvec * PT::kElems;
-    size_t tb, te;
-    shareOf(count - tailStart, P, a.rank, tb, te);
-    for (size_t i = tailStart + tb + tid; i < tailStart + te; i += nthreads) {
-      using A = typename AccType<T>::type;
-      A acc = toAcc<T>(static_cast<const T*>(bufs.p[0])[i]);
-      for (int r = 1; r < P; r++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(bufs.p[r])[i]), DevOp::SUM);
-      if (scale != 1.0f) acc = scaleAcc(acc, scale);
-      const T res = fromAcc<T, A>(acc);
-      for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = res;
-    }
-  }
+  allreduceTailInPlace<T>(bufs, P, a.rank, nvec * PT::kElems, count, DevOp::SUM, scale, tid, nthreads);
   if (blockBarrier(a, e + 2) && extra.n > 0) fanOutLocalShares<T>(mine, extra, nvec, count, P, tid, nthreads);
   retire(a, 2, 0);
 }
@@ -667,42 +563,9 @@ hybridAllreduceKernel(CommArgs a, char* mcBase, PeerPtrs bufs, size_t count, flo
     char* peer[P];
 #pragma unroll
     for (int i = 0; i < P; i++) peer[i] = static_cast<char*>(bufs.p[(a.rank + i) % P]);
-    for (size_t v0 = vb + tid; v0 < ve; v0 += nthreads * UP) {
-      Pack16 p[UP][P];
-#pragma unroll
-      for (int u = 0; u < UP; u++) {
-        const size_t v = v0 + static_cast<size_t>(u) * nthreads;
-        if (v < ve) {
-#pragma unroll
-          for (int i = 0; i < P; i++) p[u][i] = ld128_stream(peer[i] + v * 16);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < UP; u++) {
-        const size_t v = v0 + static_cast<size_t>(u) * nthreads;
-        if (v < ve) {
-          typename PT::AccPack acc = PT::widen(p[u][0]);
-#pragma unroll
-          for (int i = 1; i < P; i++) PT::combine(acc, p[u][i], DevOp::SUM);
-          if (scale != 1.0f) PT::scale(acc, scale);
-          const Pack16 res = PT::narrow(acc);
-#pragma unroll
-          for (int i = 0; i < P; i++) st128_stream(peer[i] + v * 16, res);
-        }
-      }
-    }
+    peerAllreducePacks<T, P, UP>(peer, P, vb, ve, DevOp::SUM, scale, tid, nthreads);
     // sub-pack tail: peer-to-peer group, split like the two-shot tail
-    const size_t tailStart = nvec * PT::kElems;
-    size_t tb, te;
-    shareOf(count - tailStart, P, a.rank, tb, te);
-    for (size_t i = tailStart + tb + tid; i < tailStart + te; i += nthreads) {
-      using A = typename AccType<T>::type;
-      A acc = toAcc<T>(static_cast<const T*>(bufs.p[0])[i]);
-      for (int r = 1; r < P; r++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(bufs.p[r])[i]), DevOp::SUM);
-      if (scale != 1.0f) acc = scaleAcc(acc, scale);
-      const T res = fromAcc<T, A>(acc);
-      for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = res;
-    }
+    allreduceTailInPlace<T>(bufs, P, a.rank, nvec * PT::kElems, count, DevOp::SUM, scale, tid, nthreads);
   }
   blockBarrier(a, e + 2);
   retire(a, 2, 0);
@@ -764,10 +627,10 @@ castAllreduceKernel(CommArgs a, PeerPtrs ins, char* mcIn, PeerPtrs outs, size_t 
     size_t tb, te;
     shareOf(count - tailStart, P, a.rank, tb, te);
     for (size_t i = tailStart + tb + tid; i < tailStart + te; i += nthreads) {
-      float acc = II::toFloat(static_cast<const TI*>(ins.p[0])[i]);
-      for (int r = 1; r < P; r++) acc = applyOp<float>(acc, II::toFloat(static_cast<const TI*>(ins.p[r])[i]), op);
+      float acc = toAcc<TI>(static_cast<const TI*>(ins.p[0])[i]);
+      for (int r = 1; r < P; r++) acc = applyOp<float>(acc, toAcc<TI>(static_cast<const TI*>(ins.p[r])[i]), op);
       acc *= scale;
-      for (int r = 0; r < P; r++) static_cast<TO*>(outs.p[r])[i] = OI::fromFloat(acc);
+      for (int r = 0; r < P; r++) static_cast<TO*>(outs.p[r])[i] = fromAcc<TO>(acc);
     }
   }
   blockBarrier(a, e + 2);
@@ -777,33 +640,6 @@ castAllreduceKernel(CommArgs a, PeerPtrs ins, char* mcIn, PeerPtrs outs, size_t 
 // ---- host-side launchers ----------------------------------------------------------------
 
 namespace {
-
-template <typename F>
-void dispatchType(DataType dt, F&& f) {
-  switch (dt) {
-    case DataType::INT8: f(int8_t{}); break;
-    case DataType::UINT8: f(uint8_t{}); break;
-    case DataType::INT16: f(int16_t{}); break;
-    case DataType::INT32: f(int32_t{}); break;
-    case DataType::UINT32: f(uint32_t{}); break;
-    case DataType::INT64: f((long long){}); break;
-    case DataType::UINT64: f((unsigned long long){}); break;
-    case DataType::FLOAT32: f(float{}); break;
-    case DataType::FLOAT64: f(double{}); break;
-    case DataType::FLOAT16: f(__half{}); break;
-    case DataType::BFLOAT16: f(__nv_bfloat16{}); break;
-  }
-}
-
-template <typename T>
-constexpr bool isHotType() {
-  return std::is_same<T, float>::value || std::is_same<T, __half>::value || std::is_same<T, __nv_bfloat16>::value;
-}
-
-template <typename K>
-const void* fn(K kernel) {
-  return reinterpret_cast<const void*>(kernel);
-}
 
 // The instantiation of the two-shot kernel for (T, P, unroll); unroll 0 = default for P.
 template <typename T>
@@ -829,58 +665,80 @@ const void* twoShotFn(int P, int unroll) {
 
 template <typename T>
 const void* nvlsFn(int unroll) {
-  if (unroll == 2) return fn(nvlsAllreduceKernel<T, 2>);
-  if (unroll == 8) return fn(nvlsAllreduceKernel<T, 8>);
-  return fn(nvlsAllreduceKernel<T, 4>);
+  if constexpr (isHotType<T>()) {
+    if (unroll == 2) return fn(nvlsAllreduceKernel<T, 2>);
+    if (unroll == 8) return fn(nvlsAllreduceKernel<T, 8>);
+    return fn(nvlsAllreduceKernel<T, 4>);
+  }
+  return nullptr;
 }
 
-void launch(const void* kernel, int blocks, int threads, void** args, cudaStream_t stream) {
-  cudaLaunchKernel(kernel, dim3(static_cast<unsigned>(blocks)), dim3(static_cast<unsigned>(threads)), args, 0, stream);
+template <typename T>
+const void* hybridFn(int P) {
+  if constexpr (isHotType<T>()) {
+    switch (P) {
+      case 2: return fn(hybridAllreduceKernel<T, 2>);
+      case 4: return fn(hybridAllreduceKernel<T, 4>);
+      case 8: return fn(hybridAllreduceKernel<T, 8>);
+      default: break;
+    }
+  }
+  return nullptr;
+}
+
+// LL allreduce: same dtype in and out, or one of the cast epilogue's conversions.
+const void* llKernelFor(DataType dt, DataType outDt) {
+  if (dt != outDt) {
+    return dispatchCast(dt, outDt, [](auto ti, auto to) { return fn(llAllreduceKernel<decltype(ti), decltype(to)>); });
+  }
+  return dispatchType(dt, [](auto t) { return fn(llAllreduceKernel<decltype(t), decltype(t)>); });
+}
+
+const void* oneShotKernelFor(DataType dt, bool push) {
+  return dispatchType(dt, [&](auto t) {
+    using T = decltype(t);
+    return push ? fn(oneShotPushAllreduceKernel<T>) : fn(oneShotAllreduceKernel<T>);
+  });
+}
+
+const void* llReduceScatterKernelFor(DataType dt) {
+  return dispatchType(dt, [](auto t) { return fn(llReduceScatterKernel<decltype(t)>); });
 }
 
 }  // namespace
 
-// Force-load every kernel of this file. With CUDA's lazy module loading the first
-// launch of a kernel may have to synchronise the context; if a peer rank on the same
-// device is already spinning inside its collective kernel that launch never happens
-// (documented lazy-loading deadlock for kernels that assume concurrency).
-namespace {
-void touch(const void* kernel) {
-  cudaFuncAttributes attr;
-  cudaFuncGetAttributes(&attr, kernel);
+const void* twoShotKernelFor(DataType dt, int nranks, int unroll) {
+  return dispatchType(dt, [&](auto t) { return twoShotFn<decltype(t)>(nranks, unroll); });
 }
-}  // namespace
 
+const void* nvlsKernelFor(DataType dt, int unroll) {
+  return dispatchType(dt, [&](auto t) { return nvlsFn<decltype(t)>(unroll); });
+}
+
+const void* hybridKernelFor(DataType dt, int nranks) {
+  return dispatchType(dt, [&](auto t) { return hybridFn<decltype(t)>(nranks); });
+}
+
+const void* castKernelFor(DataType in, DataType out) {
+  return dispatchCast(in, out, [](auto ti, auto to) { return fn(castAllreduceKernel<decltype(ti), decltype(to)>); });
+}
+
+// Force-load every kernel of this file (see touch()).
 void preloadAllreduceKernels() {
   touch(fn(barrierKernel));
-  for (DataType dt : {DataType::INT8, DataType::UINT8, DataType::INT16, DataType::INT32, DataType::UINT32, DataType::INT64,
-                      DataType::UINT64, DataType::FLOAT32, DataType::FLOAT64, DataType::FLOAT16, DataType::BFLOAT16}) {
-    dispatchType(dt, [&](auto tag) {
-      using T = decltype(tag);
-      touch(fn(llAllreduceKernel<T, T>));
-      touch(fn(llReduceScatterKernel<T>));
-      touch(fn(oneShotAllreduceKernel<T>));
-      touch(fn(oneShotPushAllreduceKernel<T>));
-      touch(twoShotFn<T>(0, 0));
-      if constexpr (isHotType<T>()) {
-        for (int P : {2, 4, 8}) {
-          for (int u : {1, 2, 4, 8}) touch(twoShotFn<T>(P, u));
-        }
-        for (int u : {2, 4, 8}) touch(nvlsFn<T>(u));
-      }
-    });
+  for (DataType dt : kAllDataTypes) {
+    touch(llReduceScatterKernelFor(dt));
+    for (bool push : {false, true}) touch(oneShotKernelFor(dt, push));
+    for (int P : {0, 2, 4, 8}) {
+      for (int u : {0, 1, 2, 4, 8}) touch(twoShotKernelFor(dt, P, u));
+      touch(hybridKernelFor(dt, P));
+    }
+    for (int u : {2, 4, 8}) touch(nvlsKernelFor(dt, u));
+    for (DataType outDt : kAllDataTypes) {
+      touch(llKernelFor(dt, outDt));
+      touch(castKernelFor(dt, outDt));
+    }
   }
-  for (DataType dt : {DataType::FLOAT32, DataType::FLOAT16, DataType::BFLOAT16}) {
-    for (int P : {2, 4, 8}) touch(hybridKernelFor(dt, P));
-  }
-  touch(fn(llAllreduceKernel<float, __half>));
-  touch(fn(llAllreduceKernel<float, __nv_bfloat16>));
-  touch(fn(llAllreduceKernel<__half, float>));
-  touch(fn(llAllreduceKernel<__nv_bfloat16, float>));
-  touch(fn(castAllreduceKernel<float, __half>));
-  touch(fn(castAllreduceKernel<float, __nv_bfloat16>));
-  touch(fn(castAllreduceKernel<__half, float>));
-  touch(fn(castAllreduceKernel<__nv_bfloat16, float>));
   cudaGetLastError();
 }
 
@@ -905,70 +763,42 @@ bool castSupported(DataType in, DataType out) {
 void launchLLAllreduce(const CommArgs& a, const void* in, void* out, size_t count, DataType dt, DataType outDt,
                        ReduceOp op, float scale, const PeerPtrs& ll, size_t srcStride, size_t parityStride,
                        const LocalPtrs& extra, int blocks, int threads, cudaStream_t stream) {
-  const DevOp dop = static_cast<DevOp>(op);
-#define GLB_LL(TI, TO)                                                                                              \
-  llAllreduceKernel<TI, TO><<<blocks, threads, 0, stream>>>(a, static_cast<const TI*>(in), static_cast<TO*>(out), \
-                                                           count, dop, scale, ll, static_cast<char*>(ll.p[a.rank]), \
-                                                           srcStride, parityStride, extra)
-  if (dt != outDt) {
-    if (dt == DataType::FLOAT32 && outDt == DataType::FLOAT16) GLB_LL(float, __half);
-    else if (dt == DataType::FLOAT32 && outDt == DataType::BFLOAT16) GLB_LL(float, __nv_bfloat16);
-    else if (dt == DataType::FLOAT16 && outDt == DataType::FLOAT32) GLB_LL(__half, float);
-    else if (dt == DataType::BFLOAT16 && outDt == DataType::FLOAT32) GLB_LL(__nv_bfloat16, float);
-    return;
-  }
-  dispatchType(dt, [&](auto tag) {
-    using T = decltype(tag);
-    GLB_LL(T, T);
-  });
-#undef GLB_LL
+  const void* k = llKernelFor(dt, outDt);
+  if (k == nullptr) return;
+  CommArgs ca = a;
+  DevOp dop = static_cast<DevOp>(op);
+  PeerPtrs pl = ll;
+  char* myLL = static_cast<char*>(ll.p[a.rank]);
+  LocalPtrs ex = extra;
+  void* args[] = {&ca, &in, &out, &count, &dop, &scale, &pl, &myLL, &srcStride, &parityStride, &ex};
+  launchKernel(k, blocks, threads, args, stream);
 }
 
 void launchLLReduceScatter(const CommArgs& a, const void* in, void* out, size_t perRank, DataType dt, ReduceOp op,
                            float scale, const PeerPtrs& ll, size_t srcStride, size_t parityStride, int blocks, int threads,
                            cudaStream_t stream) {
-  dispatchType(dt, [&](auto tag) {
-    using T = decltype(tag);
-    llReduceScatterKernel<T><<<blocks, threads, 0, stream>>>(a, static_cast<const T*>(in), static_cast<T*>(out), perRank,
-                                                            static_cast<DevOp>(op), scale, ll,
-                                                            static_cast<char*>(ll.p[a.rank]), srcStride, parityStride);
-  });
+  CommArgs ca = a;
+  DevOp dop = static_cast<DevOp>(op);
+  PeerPtrs pl = ll;
+  char* myLL = static_cast<char*>(ll.p[a.rank]);
+  void* args[] = {&ca, &in, &out, &perRank, &dop, &scale, &pl, &myLL, &srcStride, &parityStride};
+  launchKernel(llReduceScatterKernelFor(dt), blocks, threads, args, stream);
 }
 
 void launchOneShotAllreduce(const CommArgs& a, const void* in, void* out, size_t count, DataType dt, ReduceOp op,
                             float scale, const PeerPtrs& stage, size_t halfBytes, const LocalPtrs& extra, int blocks,
                             cudaStream_t stream) {
   // Push while every rank's copy fits a slot (half / P), else pull.
-  const size_t slotBytes = (halfBytes / static_cast<size_t>(a.nranks)) / 16 * 16;
+  size_t slotBytes = (halfBytes / static_cast<size_t>(a.nranks)) / 16 * 16;
   const size_t padded = (count * elementSize(dt) + 15) / 16 * 16;
   const bool push = padded <= slotBytes && oneShotPushEnabled();
-  dispatchType(dt, [&](auto tag) {
-    using T = decltype(tag);
-    if (push) {
-      oneShotPushAllreduceKernel<T><<<blocks, kThreads, 0, stream>>>(a, static_cast<const T*>(in), static_cast<T*>(out),
-                                                                     count, static_cast<DevOp>(op), scale, stage,
-                                                                     halfBytes, slotBytes, extra);
-    } else {
-      oneShotAllreduceKernel<T><<<blocks, kThreads, 0, stream>>>(a, static_cast<const T*>(in), static_cast<T*>(out),
-                                                                 count, static_cast<DevOp>(op), scale, stage, halfBytes,
-                                                                 extra);
-    }
-  });
-}
-
-const void* twoShotKernelFor(DataType dt, int nranks, int unroll) {
-  const void* k = nullptr;
-  dispatchType(dt, [&](auto tag) { k = twoShotFn<decltype(tag)>(nranks, unroll); });
-  return k;
-}
-
-const void* nvlsKernelFor(DataType dt, int unroll) {
-  switch (dt) {
-    case DataType::FLOAT32: return nvlsFn<float>(unroll);
-    case DataType::FLOAT16: return nvlsFn<__half>(unroll);
-    case DataType::BFLOAT16: return nvlsFn<__nv_bfloat16>(unroll);
-    default: return nullptr;
-  }
+  CommArgs ca = a;
+  DevOp dop = static_cast<DevOp>(op);
+  PeerPtrs ps = stage;
+  LocalPtrs ex = extra;
+  void* pushArgs[] = {&ca, &in, &out, &count, &dop, &scale, &ps, &halfBytes, &slotBytes, &ex};
+  void* pullArgs[] = {&ca, &in, &out, &count, &dop, &scale, &ps, &halfBytes, &ex};
+  launchKernel(oneShotKernelFor(dt, push), blocks, kThreads, push ? pushArgs : pullArgs, stream);
 }
 
 void launchTwoShotAllreduce(const CommArgs& a, const PeerPtrs& bufs, size_t count, DataType dt, ReduceOp op,
@@ -979,7 +809,7 @@ void launchTwoShotAllreduce(const CommArgs& a, const PeerPtrs& bufs, size_t coun
   PeerPtrs pb = bufs;
   LocalPtrs ex = extra;
   void* args[] = {&ca, &pb, &count, &dop, &scale, &vectorOk, &ex};
-  launch(twoShotKernelFor(dt, a.nranks, cfg.unroll), cfg.blocks, kThreads, args, stream);
+  launchKernel(twoShotKernelFor(dt, a.nranks, cfg.unroll), cfg.blocks, kThreads, args, stream);
 }
 
 bool nvlsSupports(DataType dt, ReduceOp op) {
@@ -995,28 +825,7 @@ void launchNvlsAllreduce(const CommArgs& a, void* mcPtr, const PeerPtrs& bufs, s
   PeerPtrs pb = bufs;
   LocalPtrs ex = extra;
   void* args[] = {&ca, &mc, &pb, &count, &scale, &ex};
-  launch(k, cfg.blocks, kThreads, args, stream);
-}
-
-namespace {
-template <typename T>
-const void* hybridFn(int P) {
-  switch (P) {
-    case 2: return fn(hybridAllreduceKernel<T, 2>);
-    case 4: return fn(hybridAllreduceKernel<T, 4>);
-    case 8: return fn(hybridAllreduceKernel<T, 8>);
-    default: return nullptr;
-  }
-}
-}  // namespace
-
-const void* hybridKernelFor(DataType dt, int nranks) {
-  switch (dt) {
-    case DataType::FLOAT32: return hybridFn<float>(nranks);
-    case DataType::FLOAT16: return hybridFn<__half>(nranks);
-    case DataType::BFLOAT16: return hybridFn<__nv_bfloat16>(nranks);
-    default: return nullptr;
-  }
+  launchKernel(k, cfg.blocks, kThreads, args, stream);
 }
 
 void launchHybridAllreduce(const CommArgs& a, void* mcPtr, const PeerPtrs& bufs, size_t count, DataType dt, float scale,
@@ -1027,15 +836,7 @@ void launchHybridAllreduce(const CommArgs& a, void* mcPtr, const PeerPtrs& bufs,
   char* mc = static_cast<char*>(mcPtr);
   PeerPtrs pb = bufs;
   void* args[] = {&ca, &mc, &pb, &count, &scale, &nvlsBlocks, &p2pPermille};
-  launch(k, blocks, kThreads, args, stream);
-}
-
-const void* castKernelFor(DataType in, DataType out) {
-  if (in == DataType::FLOAT32 && out == DataType::FLOAT16) return fn(castAllreduceKernel<float, __half>);
-  if (in == DataType::FLOAT32 && out == DataType::BFLOAT16) return fn(castAllreduceKernel<float, __nv_bfloat16>);
-  if (in == DataType::FLOAT16 && out == DataType::FLOAT32) return fn(castAllreduceKernel<__half, float>);
-  if (in == DataType::BFLOAT16 && out == DataType::FLOAT32) return fn(castAllreduceKernel<__nv_bfloat16, float>);
-  return nullptr;
+  launchKernel(k, blocks, kThreads, args, stream);
 }
 
 void launchCastAllreduce(const CommArgs& a, const PeerPtrs& ins, void* mcIn, const PeerPtrs& outs, size_t count,
@@ -1048,7 +849,7 @@ void launchCastAllreduce(const CommArgs& a, const PeerPtrs& ins, void* mcIn, con
   char* mc = static_cast<char*>(mcIn);
   DevOp dop = static_cast<DevOp>(op);
   void* args[] = {&ca, &pi, &mc, &po, &count, &dop, &scale, &vectorOk};
-  launch(k, blocks, kThreads, args, stream);
+  launchKernel(k, blocks, kThreads, args, stream);
 }
 
 }  // namespace cuda

@@ -5,18 +5,13 @@
 // alias exists). None of these has a CUDA variant in the reference (SURVEY §0.6).
 #include "glb/cuda/bulk_copy.cuh"
 #include "glb/cuda/device_common.cuh"
+#include "glb/cuda/dispatch.cuh"
 #include "glb/cuda/kernels.h"
 
 namespace glb {
 namespace cuda {
 
 namespace {
-
-__device__ __forceinline__ void shareOfB(size_t n, int parts, int r, size_t& begin, size_t& end) {
-  const size_t base = n / parts, rem = n % parts;
-  begin = r * base + (static_cast<size_t>(r) < rem ? r : rem);
-  end = begin + base + (static_cast<size_t>(r) < rem ? 1 : 0);
-}
 
 template <typename W>
 __device__ __forceinline__ void gridCopyWords(char* dst, const char* src, size_t bytes, size_t tid, size_t nthreads) {
@@ -293,7 +288,7 @@ broadcastKernel(CommArgs a, PeerPtrs bufs, char* mc, size_t bytes, int root, int
       for (int i = 1; i < P; i++) {
         const int dst = (root + i) % P;
         size_t b, en;
-        shareOfB(units, P, dst, b, en);
+        shareOf(units, P, dst, b, en);
         gridCopy(static_cast<char*>(bufs.p[dst]) + b * 16, static_cast<const char*>(bufs.p[root]) + b * 16,
                  (en - b) * 16, vec, tid, nthreads);
       }
@@ -311,7 +306,7 @@ broadcastKernel(CommArgs a, PeerPtrs bufs, char* mc, size_t bytes, int root, int
     // owns to all ranks that still miss it, i.e. everyone but itself and the root.
     {
       size_t b, en;
-      shareOfB(units, P, a.rank, b, en);
+      shareOf(units, P, a.rank, b, en);
       const char* src = static_cast<const char*>(bufs.p[a.rank]) + b * 16;
       const size_t nvec = vec ? (en - b) : 0;
       for (size_t v = tid; v < nvec; v += nthreads) {
@@ -561,8 +556,7 @@ reducePullKernel(CommArgs a, PeerPtrs ins, char* mcIn, T* __restrict__ out, EArg
   const size_t nvec = v16 ? len / PT::kElems : 0;
   const size_t byteOff = off * sizeof(T);
   if (useMc && v16) {
-    if constexpr (std::is_same<T, float>::value || std::is_same<T, __half>::value ||
-                  std::is_same<T, __nv_bfloat16>::value) {
+    if constexpr (isHotType<T>()) {
       constexpr int U = 4;
       for (size_t v0 = tid; v0 < nvec; v0 += nthreads * U) {
         Pack16 r[U];
@@ -575,11 +569,7 @@ reducePullKernel(CommArgs a, PeerPtrs ins, char* mcIn, T* __restrict__ out, EArg
         for (int u = 0; u < U; u++) {
           const size_t v = v0 + u * nthreads;
           if (v < nvec) {
-            if (scale != 1.0f) {
-              typename PT::AccPack acc = PT::widen(r[u]);
-              PT::scale(acc, scale);
-              r[u] = PT::narrow(acc);
-            }
+            if (scale != 1.0f) r[u] = scalePack<T>(r[u], scale);
             st128(reinterpret_cast<char*>(out) + v * 16, r[u]);
           }
         }
@@ -631,22 +621,22 @@ reducePullKernel(CommArgs a, PeerPtrs ins, char* mcIn, T* __restrict__ out, EArg
 }
 
 namespace {
+// The instantiation of the reduce pull kernel for (T, P): rank-count specialisations of the
+// hot types with their unroll, the generic kernel otherwise.
 template <typename T>
-void launchReducePullT(const CommArgs& a, const PeerPtrs& ins, char* mc, void* out, const EArgs& ea, DevOp dop,
-                       float scale, bool vec, bool useMc, int blocks, cudaStream_t stream) {
-  constexpr bool hot = std::is_same<T, float>::value || std::is_same<T, __half>::value ||
-                       std::is_same<T, __nv_bfloat16>::value;
-  if constexpr (hot) {
-    switch (a.nranks) {
-      case 2: reducePullKernel<T, 2, 4><<<blocks, kThreads, 0, stream>>>(a, ins, mc, static_cast<T*>(out), ea, dop, scale, vec, useMc); return;
-      case 4: reducePullKernel<T, 4, 2><<<blocks, kThreads, 0, stream>>>(a, ins, mc, static_cast<T*>(out), ea, dop, scale, vec, useMc); return;
-      case 8: reducePullKernel<T, 8, 2><<<blocks, kThreads, 0, stream>>>(a, ins, mc, static_cast<T*>(out), ea, dop, scale, vec, useMc); return;
-      default: break;
-    }
+const void* reducePullFn(int P) {
+  if constexpr (isHotType<T>()) {
+    if (P == 2) return fn(reducePullKernel<T, 2, 4>);
+    if (P == 4) return fn(reducePullKernel<T, 4, 2>);
+    if (P == 8) return fn(reducePullKernel<T, 8, 2>);
   }
-  reducePullKernel<T, 0, 1><<<blocks, kThreads, 0, stream>>>(a, ins, mc, static_cast<T*>(out), ea, dop, scale, vec, useMc);
+  return fn(reducePullKernel<T, 0, 1>);
 }
 }  // namespace
+
+const void* reducePullKernelPtr(DataType dt, int nranks) {
+  return dispatchType(dt, [&](auto t) { return reducePullFn<decltype(t)>(nranks); });
+}
 
 void launchReducePull(const CommArgs& a, const PeerPtrs& ins, void* mcIn, void* out, const size_t* elemOff,
                       const size_t* elemLen, DataType dt, ReduceOp op, float scale, bool vec, bool useMc, int blocks,
@@ -656,26 +646,12 @@ void launchReducePull(const CommArgs& a, const PeerPtrs& ins, void* mcIn, void* 
     ea.off[i] = i < a.nranks ? elemOff[i] : 0;
     ea.len[i] = i < a.nranks ? elemLen[i] : 0;
   }
-  const DevOp dop = static_cast<DevOp>(op);
+  CommArgs ca = a;
+  PeerPtrs pi = ins;
   char* mc = static_cast<char*>(mcIn);
-#define GLB_CASE(E, T)                                                              \
-  case DataType::E:                                                                 \
-    launchReducePullT<T>(a, ins, mc, out, ea, dop, scale, vec, useMc, blocks, stream);     \
-    break;
-  switch (dt) {
-    GLB_CASE(INT8, int8_t)
-    GLB_CASE(UINT8, uint8_t)
-    GLB_CASE(INT16, int16_t)
-    GLB_CASE(INT32, int32_t)
-    GLB_CASE(UINT32, uint32_t)
-    GLB_CASE(INT64, long long)
-    GLB_CASE(UINT64, unsigned long long)
-    GLB_CASE(FLOAT32, float)
-    GLB_CASE(FLOAT64, double)
-    GLB_CASE(FLOAT16, __half)
-    GLB_CASE(BFLOAT16, __nv_bfloat16)
-  }
-#undef GLB_CASE
+  DevOp dop = static_cast<DevOp>(op);
+  void* args[] = {&ca, &pi, &mc, &out, &ea, &dop, &scale, &vec, &useMc};
+  launchKernel(reducePullKernelPtr(dt, a.nranks), blocks, kThreads, args, stream);
 }
 
 
@@ -755,62 +731,22 @@ void launchLLExchange(const CommArgs& a, const void* in, void* out, size_t bytes
                                                    ll, srcStride, parityStride);
 }
 
-const void* broadcastKernelPtr() { return reinterpret_cast<const void*>(broadcastKernel); }
-const void* gatherPushKernelPtr() { return reinterpret_cast<const void*>(gatherPushKernel); }
-const void* gatherBulkKernelPtr() { return reinterpret_cast<const void*>(gatherBulkKernel); }
-const void* alltoallPushKernelPtr() { return reinterpret_cast<const void*>(alltoallPushKernel); }
-const void* reducePullKernelPtr(DataType dt, int nranks) {
-#define GLB_RP(E, T)                                                                                   \
-  case DataType::E: {                                                                                  \
-    constexpr bool hot = std::is_same<T, float>::value || std::is_same<T, __half>::value ||            \
-                         std::is_same<T, __nv_bfloat16>::value;                                        \
-    if constexpr (hot) {                                                                               \
-      if (nranks == 2) return reinterpret_cast<const void*>(reducePullKernel<T, 2, 4>);                \
-      if (nranks == 4) return reinterpret_cast<const void*>(reducePullKernel<T, 4, 2>);                \
-      if (nranks == 8) return reinterpret_cast<const void*>(reducePullKernel<T, 8, 2>);                \
-    }                                                                                                  \
-    return reinterpret_cast<const void*>(reducePullKernel<T, 0, 1>);                                   \
-  }
-  switch (dt) {
-    GLB_RP(INT8, int8_t)
-    GLB_RP(UINT8, uint8_t)
-    GLB_RP(INT16, int16_t)
-    GLB_RP(INT32, int32_t)
-    GLB_RP(UINT32, uint32_t)
-    GLB_RP(INT64, long long)
-    GLB_RP(UINT64, unsigned long long)
-    GLB_RP(FLOAT32, float)
-    GLB_RP(FLOAT64, double)
-    GLB_RP(FLOAT16, __half)
-    GLB_RP(BFLOAT16, __nv_bfloat16)
-  }
-#undef GLB_RP
-  return nullptr;
-}
+const void* broadcastKernelPtr() { return fn(broadcastKernel); }
+const void* gatherPushKernelPtr() { return fn(gatherPushKernel); }
+const void* gatherBulkKernelPtr() { return fn(gatherBulkKernel); }
+const void* alltoallPushKernelPtr() { return fn(alltoallPushKernel); }
 
 void preloadCollectiveKernels() {
-  auto touch = [](const void* k) {
-    cudaFuncAttributes attr;
-    cudaFuncGetAttributes(&attr, k);
-  };
-  touch(reinterpret_cast<const void*>(broadcastKernel));
-  touch(reinterpret_cast<const void*>(gatherPushKernel));
-  cudaFuncSetAttribute(reinterpret_cast<const void*>(gatherBulkKernel), cudaFuncAttributeMaxDynamicSharedMemorySize,
+  touch(fn(broadcastKernel));
+  touch(fn(gatherPushKernel));
+  cudaFuncSetAttribute(fn(gatherBulkKernel), cudaFuncAttributeMaxDynamicSharedMemorySize,
                        static_cast<int>(kBulkSmemBytes));
-  touch(reinterpret_cast<const void*>(gatherBulkKernel));
-  touch(reinterpret_cast<const void*>(alltoallPushKernel));
-  touch(reinterpret_cast<const void*>(llExchangeKernel));
-#define GLB_TOUCH_RP(T) touch(reinterpret_cast<const void*>(reducePullKernel<T, 0, 1>));
-  GLB_TOUCH_RP(int8_t) GLB_TOUCH_RP(uint8_t) GLB_TOUCH_RP(int16_t) GLB_TOUCH_RP(int32_t) GLB_TOUCH_RP(uint32_t)
-  GLB_TOUCH_RP(long long) GLB_TOUCH_RP(unsigned long long) GLB_TOUCH_RP(float) GLB_TOUCH_RP(double)
-  GLB_TOUCH_RP(__half) GLB_TOUCH_RP(__nv_bfloat16)
-#undef GLB_TOUCH_RP
-#define GLB_TOUCH_HOT(T)                                                   \
-  touch(reinterpret_cast<const void*>(reducePullKernel<T, 2, 4>));         \
-  touch(reinterpret_cast<const void*>(reducePullKernel<T, 4, 2>));         \
-  touch(reinterpret_cast<const void*>(reducePullKernel<T, 8, 2>));
-  GLB_TOUCH_HOT(float) GLB_TOUCH_HOT(__half) GLB_TOUCH_HOT(__nv_bfloat16)
-#undef GLB_TOUCH_HOT
+  touch(fn(gatherBulkKernel));
+  touch(fn(alltoallPushKernel));
+  touch(fn(llExchangeKernel));
+  for (DataType dt : kAllDataTypes) {
+    for (int P : {0, 2, 4, 8}) touch(reducePullKernelPtr(dt, P));
+  }
   cudaGetLastError();
 }
 

@@ -226,136 +226,6 @@ __device__ __forceinline__ T applyOp(T a, T b, DevOp op) {
   }
 }
 
-// Accumulator traits: how one 16-byte pack of T is widened, combined, narrowed.
-template <typename T>
-struct PackTraits {
-  static constexpr int kElems = 16 / sizeof(T);
-  using Acc = T;
-  struct AccPack {
-    T v[kElems];
-  };
-  __device__ static AccPack widen(const Pack16& p) {
-    AccPack a;
-    const T* t = reinterpret_cast<const T*>(&p);
-#pragma unroll
-    for (int i = 0; i < kElems; i++) a.v[i] = t[i];
-    return a;
-  }
-  __device__ static void combine(AccPack& a, const Pack16& p, DevOp op) {
-    const T* t = reinterpret_cast<const T*>(&p);
-#pragma unroll
-    for (int i = 0; i < kElems; i++) a.v[i] = applyOp<T>(a.v[i], t[i], op);
-  }
-  __device__ static Pack16 narrow(const AccPack& a) {
-    Pack16 p;
-    T* t = reinterpret_cast<T*>(&p);
-#pragma unroll
-    for (int i = 0; i < kElems; i++) t[i] = a.v[i];
-    return p;
-  }
-  __device__ static T one(const T* p) { return *p; }
-  // combineOne / scaleOne round to T after every step. Only the literal schedules use them:
-  // they store each step's partial in T by design. Fused kernels go through AccType below.
-  __device__ static T combineOne(T a, T b, DevOp op) { return applyOp<T>(a, b, op); }
-  // Epilogue: multiply the reduced value (floating types only; the host rejects a scale
-  // on integer buffers).
-  __device__ static void scale(AccPack& a, float s) {
-    if constexpr (std::is_floating_point<T>::value) {
-#pragma unroll
-      for (int i = 0; i < kElems; i++) a.v[i] = static_cast<T>(a.v[i] * s);
-    }
-  }
-  __device__ static T scaleOne(T a, float s) {
-    if constexpr (std::is_floating_point<T>::value) return static_cast<T>(a * s);
-    return a;
-  }
-};
-
-template <>
-struct PackTraits<__half> {
-  static constexpr int kElems = 8;
-  struct AccPack {
-    float v[8];
-  };
-  __device__ static AccPack widen(const Pack16& p) {
-    AccPack a;
-    const __half2* h = reinterpret_cast<const __half2*>(&p);
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-      float2 f = __half22float2(h[i]);
-      a.v[2 * i] = f.x;
-      a.v[2 * i + 1] = f.y;
-    }
-    return a;
-  }
-  __device__ static void combine(AccPack& a, const Pack16& p, DevOp op) {
-    const __half2* h = reinterpret_cast<const __half2*>(&p);
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-      float2 f = __half22float2(h[i]);
-      a.v[2 * i] = applyOp<float>(a.v[2 * i], f.x, op);
-      a.v[2 * i + 1] = applyOp<float>(a.v[2 * i + 1], f.y, op);
-    }
-  }
-  __device__ static Pack16 narrow(const AccPack& a) {
-    Pack16 p;
-    __half2* h = reinterpret_cast<__half2*>(&p);
-#pragma unroll
-    for (int i = 0; i < 4; i++) h[i] = __floats2half2_rn(a.v[2 * i], a.v[2 * i + 1]);
-    return p;
-  }
-  __device__ static __half combineOne(__half a, __half b, DevOp op) {
-    return __float2half_rn(applyOp<float>(__half2float(a), __half2float(b), op));
-  }
-  __device__ static void scale(AccPack& a, float s) {
-#pragma unroll
-    for (int i = 0; i < 8; i++) a.v[i] *= s;
-  }
-  __device__ static __half scaleOne(__half a, float s) { return __float2half_rn(__half2float(a) * s); }
-};
-
-template <>
-struct PackTraits<__nv_bfloat16> {
-  static constexpr int kElems = 8;
-  struct AccPack {
-    float v[8];
-  };
-  __device__ static AccPack widen(const Pack16& p) {
-    AccPack a;
-    // bf16 -> fp32 is a 16-bit shift.
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-      a.v[2 * i] = __uint_as_float(p.w[i] << 16);
-      a.v[2 * i + 1] = __uint_as_float(p.w[i] & 0xffff0000u);
-    }
-    return a;
-  }
-  __device__ static void combine(AccPack& a, const Pack16& p, DevOp op) {
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-      a.v[2 * i] = applyOp<float>(a.v[2 * i], __uint_as_float(p.w[i] << 16), op);
-      a.v[2 * i + 1] = applyOp<float>(a.v[2 * i + 1], __uint_as_float(p.w[i] & 0xffff0000u), op);
-    }
-  }
-  __device__ static Pack16 narrow(const AccPack& a) {
-    Pack16 p;
-    __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&p);
-#pragma unroll
-    for (int i = 0; i < 4; i++) h[i] = __floats2bfloat162_rn(a.v[2 * i], a.v[2 * i + 1]);
-    return p;
-  }
-  __device__ static __nv_bfloat16 combineOne(__nv_bfloat16 a, __nv_bfloat16 b, DevOp op) {
-    return __float2bfloat16_rn(applyOp<float>(__bfloat162float(a), __bfloat162float(b), op));
-  }
-  __device__ static void scale(AccPack& a, float s) {
-#pragma unroll
-    for (int i = 0; i < 8; i++) a.v[i] *= s;
-  }
-  __device__ static __nv_bfloat16 scaleOne(__nv_bfloat16 a, float s) {
-    return __float2bfloat16_rn(__bfloat162float(a) * s);
-  }
-};
-
 // ---- one element at a time ---------------------------------------------------------------
 // The scalar paths (sub-pack tails, unaligned buffers, uneven shares) follow the same rule as
 // the packs: widen to AccType<T>, reduce and scale there, round once with fromAcc. AccType is
@@ -404,12 +274,149 @@ __device__ __forceinline__ A scaleAcc(A x, float s) {
   return x;
 }
 
+// combineOne / scaleOne round to T after every step. Only the literal schedules use them:
+// they store each step's partial in T by design. Fused kernels round once (above).
+template <typename T>
+__device__ __forceinline__ T combineOne(T a, T b, DevOp op) {
+  using A = typename AccType<T>::type;
+  return fromAcc<T, A>(applyOp<A>(toAcc<T>(a), toAcc<T>(b), op));
+}
+template <typename T>
+__device__ __forceinline__ T scaleOne(T a, float s) {
+  return fromAcc<T>(scaleAcc(toAcc<T>(a), s));
+}
+
+// Accumulator traits: how one 16-byte pack of T is widened, combined, narrowed.
+template <typename T>
+struct PackTraits {
+  static constexpr int kElems = 16 / sizeof(T);
+  using Acc = T;
+  struct AccPack {
+    T v[kElems];
+  };
+  __device__ static AccPack widen(const Pack16& p) {
+    AccPack a;
+    const T* t = reinterpret_cast<const T*>(&p);
+#pragma unroll
+    for (int i = 0; i < kElems; i++) a.v[i] = t[i];
+    return a;
+  }
+  __device__ static void combine(AccPack& a, const Pack16& p, DevOp op) {
+    const T* t = reinterpret_cast<const T*>(&p);
+#pragma unroll
+    for (int i = 0; i < kElems; i++) a.v[i] = applyOp<T>(a.v[i], t[i], op);
+  }
+  __device__ static Pack16 narrow(const AccPack& a) {
+    Pack16 p;
+    T* t = reinterpret_cast<T*>(&p);
+#pragma unroll
+    for (int i = 0; i < kElems; i++) t[i] = a.v[i];
+    return p;
+  }
+  // Epilogue: multiply the reduced value (floating types only; the host rejects a scale
+  // on integer buffers).
+  __device__ static void scale(AccPack& a, float s) {
+    if constexpr (std::is_floating_point<T>::value) {
+#pragma unroll
+      for (int i = 0; i < kElems; i++) a.v[i] = static_cast<T>(a.v[i] * s);
+    }
+  }
+};
+
+template <>
+struct PackTraits<__half> {
+  static constexpr int kElems = 8;
+  struct AccPack {
+    float v[8];
+  };
+  __device__ static AccPack widen(const Pack16& p) {
+    AccPack a;
+    const __half2* h = reinterpret_cast<const __half2*>(&p);
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      float2 f = __half22float2(h[i]);
+      a.v[2 * i] = f.x;
+      a.v[2 * i + 1] = f.y;
+    }
+    return a;
+  }
+  __device__ static void combine(AccPack& a, const Pack16& p, DevOp op) {
+    const __half2* h = reinterpret_cast<const __half2*>(&p);
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      float2 f = __half22float2(h[i]);
+      a.v[2 * i] = applyOp<float>(a.v[2 * i], f.x, op);
+      a.v[2 * i + 1] = applyOp<float>(a.v[2 * i + 1], f.y, op);
+    }
+  }
+  __device__ static Pack16 narrow(const AccPack& a) {
+    Pack16 p;
+    __half2* h = reinterpret_cast<__half2*>(&p);
+#pragma unroll
+    for (int i = 0; i < 4; i++) h[i] = __floats2half2_rn(a.v[2 * i], a.v[2 * i + 1]);
+    return p;
+  }
+  __device__ static void scale(AccPack& a, float s) {
+#pragma unroll
+    for (int i = 0; i < 8; i++) a.v[i] *= s;
+  }
+};
+
+template <>
+struct PackTraits<__nv_bfloat16> {
+  static constexpr int kElems = 8;
+  struct AccPack {
+    float v[8];
+  };
+  __device__ static AccPack widen(const Pack16& p) {
+    AccPack a;
+    // bf16 -> fp32 is a 16-bit shift.
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      a.v[2 * i] = __uint_as_float(p.w[i] << 16);
+      a.v[2 * i + 1] = __uint_as_float(p.w[i] & 0xffff0000u);
+    }
+    return a;
+  }
+  __device__ static void combine(AccPack& a, const Pack16& p, DevOp op) {
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      a.v[2 * i] = applyOp<float>(a.v[2 * i], __uint_as_float(p.w[i] << 16), op);
+      a.v[2 * i + 1] = applyOp<float>(a.v[2 * i + 1], __uint_as_float(p.w[i] & 0xffff0000u), op);
+    }
+  }
+  __device__ static Pack16 narrow(const AccPack& a) {
+    Pack16 p;
+    __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&p);
+#pragma unroll
+    for (int i = 0; i < 4; i++) h[i] = __floats2bfloat162_rn(a.v[2 * i], a.v[2 * i + 1]);
+    return p;
+  }
+  __device__ static void scale(AccPack& a, float s) {
+#pragma unroll
+    for (int i = 0; i < 8; i++) a.v[i] *= s;
+  }
+};
+
 // ---- mixed-precision items (cast epilogue) --------------------------------------------
 // Eight consecutive elements of T as fp32 lanes: 2 x 16 B for float, 1 x 16 B for the
 // 16-bit types. Used by the kernels whose output dtype differs from the input dtype
 // (fp32 accumulate -> bf16/fp16 store, or 16-bit inputs -> fp32 result).
-template <typename T>
-struct Item8;
+template <typename T>  // __half, __nv_bfloat16
+struct Item8 {
+  static constexpr int kBytes = 16;
+  __device__ static void load(const void* p, float (&v)[8]) {
+    const auto a = PackTraits<T>::widen(ld128_stream(p));
+#pragma unroll
+    for (int i = 0; i < 8; i++) v[i] = a.v[i];
+  }
+  __device__ static void store(void* p, const float (&v)[8]) {
+    typename PackTraits<T>::AccPack a;
+#pragma unroll
+    for (int i = 0; i < 8; i++) a.v[i] = v[i];
+    st128_stream(p, PackTraits<T>::narrow(a));
+  }
+};
 template <>
 struct Item8<float> {
   static constexpr int kBytes = 32;
@@ -431,42 +438,6 @@ struct Item8<float> {
     st128_stream(p, a);
     st128_stream(static_cast<char*>(p) + 16, b);
   }
-  __device__ static float toFloat(float x) { return x; }
-  __device__ static float fromFloat(float x) { return x; }
-};
-template <>
-struct Item8<__half> {
-  static constexpr int kBytes = 16;
-  __device__ static void load(const void* p, float (&v)[8]) {
-    const auto a = PackTraits<__half>::widen(ld128_stream(p));
-#pragma unroll
-    for (int i = 0; i < 8; i++) v[i] = a.v[i];
-  }
-  __device__ static void store(void* p, const float (&v)[8]) {
-    PackTraits<__half>::AccPack a;
-#pragma unroll
-    for (int i = 0; i < 8; i++) a.v[i] = v[i];
-    st128_stream(p, PackTraits<__half>::narrow(a));
-  }
-  __device__ static float toFloat(__half x) { return __half2float(x); }
-  __device__ static __half fromFloat(float x) { return __float2half_rn(x); }
-};
-template <>
-struct Item8<__nv_bfloat16> {
-  static constexpr int kBytes = 16;
-  __device__ static void load(const void* p, float (&v)[8]) {
-    const auto a = PackTraits<__nv_bfloat16>::widen(ld128_stream(p));
-#pragma unroll
-    for (int i = 0; i < 8; i++) v[i] = a.v[i];
-  }
-  __device__ static void store(void* p, const float (&v)[8]) {
-    PackTraits<__nv_bfloat16>::AccPack a;
-#pragma unroll
-    for (int i = 0; i < 8; i++) a.v[i] = v[i];
-    st128_stream(p, PackTraits<__nv_bfloat16>::narrow(a));
-  }
-  __device__ static float toFloat(__nv_bfloat16 x) { return __bfloat162float(x); }
-  __device__ static __nv_bfloat16 fromFloat(float x) { return __float2bfloat16_rn(x); }
 };
 
 // ---- NVLS (multimem) --------------------------------------------------------------
@@ -516,20 +487,120 @@ __device__ __forceinline__ void multimemSt128(void* mc, const Pack16& v) {
                : "memory");
 }
 
-// Map the public dtype tags to device element types.
-template <DataType D>
-struct DevType;
-template <> struct DevType<DataType::INT8> { using type = int8_t; };
-template <> struct DevType<DataType::UINT8> { using type = uint8_t; };
-template <> struct DevType<DataType::INT16> { using type = int16_t; };
-template <> struct DevType<DataType::INT32> { using type = int32_t; };
-template <> struct DevType<DataType::UINT32> { using type = uint32_t; };
-template <> struct DevType<DataType::INT64> { using type = long long; };
-template <> struct DevType<DataType::UINT64> { using type = unsigned long long; };
-template <> struct DevType<DataType::FLOAT32> { using type = float; };
-template <> struct DevType<DataType::FLOAT64> { using type = double; };
-template <> struct DevType<DataType::FLOAT16> { using type = __half; };
-template <> struct DevType<DataType::BFLOAT16> { using type = __nv_bfloat16; };
+// ---- building blocks of the fused kernels ---------------------------------------------------
+
+// [begin, end) of rank r's share of n items.
+__device__ __forceinline__ void shareOf(size_t n, int parts, int r, size_t& begin, size_t& end) {
+  const size_t base = n / parts, rem = n % parts;
+  begin = r * base + (static_cast<size_t>(r) < rem ? r : rem);
+  end = begin + base + (static_cast<size_t>(r) < rem ? 1 : 0);
+}
+
+// Element groups. The barrier pairs CTA b of one rank with CTA b of every peer, so which CTA
+// touches which element must not depend on anything rank-local (such as the alignment of a
+// user pointer). The staged kernels therefore own 16-byte *groups* of elements by index; a
+// group is moved with one 128-bit access when the pointer allows it and element by element
+// otherwise (zero padded past `count`).
+template <typename T>
+__device__ __forceinline__ Pack16 loadGroup(const T* base, size_t g, size_t count, bool aligned) {
+  constexpr int K = 16 / sizeof(T);
+  const size_t i0 = g * K;
+  if (aligned && i0 + K <= count) return ld128_stream(reinterpret_cast<const char*>(base) + g * 16);
+  Pack16 p;
+  p.w[0] = p.w[1] = p.w[2] = p.w[3] = 0u;
+  T* t = reinterpret_cast<T*>(&p);
+#pragma unroll
+  for (int k = 0; k < K; k++) {
+    if (i0 + k < count) t[k] = base[i0 + k];
+  }
+  return p;
+}
+
+// kStream: the 128-bit store does not allocate in L1 (st128_stream) instead of st128.
+template <bool kStream, typename T>
+__device__ __forceinline__ void storeGroup(T* base, size_t g, size_t count, bool aligned, const Pack16& p) {
+  constexpr int K = 16 / sizeof(T);
+  const size_t i0 = g * K;
+  if (aligned && i0 + K <= count) {
+    if constexpr (kStream) {
+      st128_stream(reinterpret_cast<char*>(base) + g * 16, p);
+    } else {
+      st128(reinterpret_cast<char*>(base) + g * 16, p);
+    }
+    return;
+  }
+  const T* t = reinterpret_cast<const T*>(&p);
+#pragma unroll
+  for (int k = 0; k < K; k++) {
+    if (i0 + k < count) base[i0 + k] = t[k];
+  }
+}
+
+template <typename T>
+__device__ __forceinline__ Pack16 scalePack(const Pack16& p, float s) {
+  using PT = PackTraits<T>;
+  typename PT::AccPack acc = PT::widen(p);
+  PT::scale(acc, s);
+  return PT::narrow(acc);
+}
+
+// In place over peer pointers: pack v of the P buffers peer[0..P) is loaded from all of them,
+// reduced in peer order, scaled, rounded once and stored to all of them, for v in [vb, ve),
+// U packs per thread and trip (kSlots x U independent 128-bit loads in flight).
+template <typename T, int kSlots, int U>
+__device__ __forceinline__ void peerAllreducePacks(char* const (&peer)[kSlots], int P, size_t vb, size_t ve, DevOp op,
+                                                   float scale, size_t tid, size_t nthreads) {
+  using PT = PackTraits<T>;
+  for (size_t v0 = vb + tid; v0 < ve; v0 += nthreads * U) {
+    Pack16 p[U][kSlots];
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+      const size_t v = v0 + static_cast<size_t>(u) * nthreads;
+      if (v < ve) {
+#pragma unroll
+        for (int i = 0; i < kSlots; i++) {
+          if (i < P) p[u][i] = ld128_stream(peer[i] + v * 16);
+        }
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+      const size_t v = v0 + static_cast<size_t>(u) * nthreads;
+      if (v < ve) {
+        typename PT::AccPack acc = PT::widen(p[u][0]);
+#pragma unroll
+        for (int i = 1; i < kSlots; i++) {
+          if (i < P) PT::combine(acc, p[u][i], op);
+        }
+        if (scale != 1.0f) PT::scale(acc, scale);
+        const Pack16 res = PT::narrow(acc);
+#pragma unroll
+        for (int i = 0; i < kSlots; i++) {
+          if (i < P) st128_stream(peer[i] + v * 16, res);
+        }
+      }
+    }
+  }
+}
+
+// Element tail of the in-place allreduce (count not a multiple of the pack width, or
+// unaligned buffers): rank `rank`'s share of [tailStart, count), reduced across the P buffers
+// in AccType<T>, scaled, rounded once and stored to all P.
+template <typename T>
+__device__ __forceinline__ void allreduceTailInPlace(const PeerPtrs& bufs, int P, int rank, size_t tailStart,
+                                                     size_t count, DevOp op, float scale, size_t tid,
+                                                     size_t nthreads) {
+  using A = typename AccType<T>::type;
+  size_t tb, te;
+  shareOf(count - tailStart, P, rank, tb, te);
+  for (size_t i = tailStart + tb + tid; i < tailStart + te; i += nthreads) {
+    A acc = toAcc<T>(static_cast<const T*>(bufs.p[0])[i]);
+    for (int r = 1; r < P; r++) acc = applyOp<A>(acc, toAcc<T>(static_cast<const T*>(bufs.p[r])[i]), op);
+    if (scale != 1.0f) acc = scaleAcc(acc, scale);
+    const T res = fromAcc<T, A>(acc);
+    for (int r = 0; r < P; r++) static_cast<T*>(bufs.p[r])[i] = res;
+  }
+}
 
 }  // namespace cuda
 }  // namespace glb

@@ -15,6 +15,7 @@
 // memory (RemoteKey semantics, transport/unbound_buffer.h:128-152).
 #include "glb/cuda/bulk_copy.cuh"
 #include "glb/cuda/device_common.cuh"
+#include "glb/cuda/dispatch.cuh"
 #include "glb/cuda/kernels.h"
 
 namespace glb {
@@ -223,16 +224,14 @@ __global__ void __launch_bounds__(128) peerBulkCopyKernel(char* dst, const char*
 }
 
 void preloadP2pKernels() {
-  cudaFuncSetAttribute(reinterpret_cast<const void*>(peerBulkCopyKernel), cudaFuncAttributeMaxDynamicSharedMemorySize,
+  cudaFuncSetAttribute(fn(peerBulkCopyKernel), cudaFuncAttributeMaxDynamicSharedMemorySize,
                        static_cast<int>(kBulkSmemBytes));
-  cudaFuncAttributes attr;
-  cudaFuncGetAttributes(&attr, reinterpret_cast<const void*>(p2pKernel));
-  cudaFuncGetAttributes(&attr, reinterpret_cast<const void*>(peerCopyKernel));
-  cudaFuncGetAttributes(&attr, reinterpret_cast<const void*>(peerBulkCopyKernel));
-  cudaFuncGetAttributes(&attr, reinterpret_cast<const void*>(exchangeKernel<false>));
-  cudaFuncGetAttributes(&attr, reinterpret_cast<const void*>(exchangeKernel<true>));
-  cudaFuncSetAttribute(reinterpret_cast<const void*>(exchangeKernel<true>), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                       kBulkSmemBytes);
+  touch(fn(p2pKernel));
+  touch(fn(peerCopyKernel));
+  touch(fn(peerBulkCopyKernel));
+  touch(fn(exchangeKernel<false>));
+  touch(fn(exchangeKernel<true>));
+  cudaFuncSetAttribute(fn(exchangeKernel<true>), cudaFuncAttributeMaxDynamicSharedMemorySize, kBulkSmemBytes);
   cudaGetLastError();
 }
 

@@ -19,44 +19,11 @@
 // share in every stage, so the CTA-to-CTA flag barrier is all the synchronisation needed
 // (the CTA that reads a peer's tile is barrier-paired with the CTA that wrote it).
 #include "glb/cuda/device_common.cuh"
+#include "glb/cuda/dispatch.cuh"
 #include "glb/cuda/kernels.h"
 
 namespace glb {
 namespace cuda {
-
-namespace {
-
-template <typename T>
-__device__ __forceinline__ Pack16 loadGroupP(const T* base, size_t g, size_t count, bool aligned) {
-  constexpr int K = 16 / sizeof(T);
-  const size_t i0 = g * K;
-  if (aligned && i0 + K <= count) return ld128_stream(reinterpret_cast<const char*>(base) + g * 16);
-  Pack16 p;
-  p.w[0] = p.w[1] = p.w[2] = p.w[3] = 0u;
-  T* t = reinterpret_cast<T*>(&p);
-#pragma unroll
-  for (int k = 0; k < K; k++) {
-    if (i0 + k < count) t[k] = base[i0 + k];
-  }
-  return p;
-}
-
-template <typename T>
-__device__ __forceinline__ void storeGroupP(T* base, size_t g, size_t count, bool aligned, const Pack16& p) {
-  constexpr int K = 16 / sizeof(T);
-  const size_t i0 = g * K;
-  if (aligned && i0 + K <= count) {
-    st128_stream(reinterpret_cast<char*>(base) + g * 16, p);
-    return;
-  }
-  const T* t = reinterpret_cast<const T*>(&p);
-#pragma unroll
-  for (int k = 0; k < K; k++) {
-    if (i0 + k < count) base[i0 + k] = t[k];
-  }
-}
-
-}  // namespace
 
 template <typename T, bool MC, int NR>
 __global__ void __launch_bounds__(kThreads)
@@ -103,11 +70,7 @@ pipelinedAllreduceKernel(CommArgs a, const T* in, T* out, size_t count, DevOp op
             for (int u = 0; u < U; u++) {
               const size_t o = o0 + static_cast<size_t>(u) * xn;
               if (o < T_) {
-                if (scale != 1.0f) {
-                  typename PT::AccPack acc = PT::widen(r[u]);
-                  PT::scale(acc, scale);
-                  r[u] = PT::narrow(acc);
-                }
+                if (scale != 1.0f) r[u] = scalePack<T>(r[u], scale);
                 multimemSt128(mc + o * 16, r[u]);
               }
             }
@@ -122,36 +85,7 @@ pipelinedAllreduceKernel(CommArgs a, const T* in, T* out, size_t count, DevOp op
           for (int q = 0; q < kSlots; q++) {
             peer[q] = q < P ? static_cast<char*>(stage.p[(a.rank + q) % P]) + slot + w0 * 16 : nullptr;
           }
-          for (size_t o0 = xt; o0 < T_; o0 += static_cast<size_t>(xn) * U) {
-            Pack16 v[U][kSlots];
-#pragma unroll
-            for (int u = 0; u < U; u++) {
-              const size_t o = o0 + static_cast<size_t>(u) * xn;
-              if (o < T_) {
-#pragma unroll
-                for (int q = 0; q < kSlots; q++) {
-                  if (q < P) v[u][q] = ld128_stream(peer[q] + o * 16);
-                }
-              }
-            }
-#pragma unroll
-            for (int u = 0; u < U; u++) {
-              const size_t o = o0 + static_cast<size_t>(u) * xn;
-              if (o < T_) {
-                typename PT::AccPack acc = PT::widen(v[u][0]);
-#pragma unroll
-                for (int q = 1; q < kSlots; q++) {
-                  if (q < P) PT::combine(acc, v[u][q], op);
-                }
-                if (scale != 1.0f) PT::scale(acc, scale);
-                const Pack16 res = PT::narrow(acc);
-#pragma unroll
-                for (int q = 0; q < kSlots; q++) {
-                  if (q < P) st128_stream(peer[q] + o * 16, res);
-                }
-              }
-            }
-          }
+          peerAllreducePacks<T, kSlots, U>(peer, P, 0, T_, op, scale, xt, xn);
         }
       }
     } else {
@@ -175,8 +109,8 @@ pipelinedAllreduceKernel(CommArgs a, const T* in, T* out, size_t count, DevOp op
 #pragma unroll
           for (int u = 0; u < CU; u++) {
             if (g[u] < ngroups) {
-              storeGroupP(out, g[u], count, aligned, p[u]);
-              for (int k = 0; k < extra.n; k++) storeGroupP(static_cast<T*>(extra.p[k]), g[u], count, aligned, p[u]);
+              storeGroup<true>(out, g[u], count, aligned, p[u]);
+              for (int k = 0; k < extra.n; k++) storeGroup<true>(static_cast<T*>(extra.p[k]), g[u], count, aligned, p[u]);
             }
           }
         }
@@ -194,11 +128,11 @@ pipelinedAllreduceKernel(CommArgs a, const T* in, T* out, size_t count, DevOp op
             w[u] = j < PT_ ? (((j >> tileShift) * G + b) << tileShift) + (j & (T_ - 1)) : chunkVecs;
             const size_t g = g0 + w[u];
             if (w[u] < chunkVecs && g < ngroups) {
-              p[u] = loadGroupP(in, g, count, aligned);
+              p[u] = loadGroup(in, g, count, aligned);
               if (extra.n > 0) {
                 typename PT::AccPack acc = PT::widen(p[u]);
                 for (int k = 0; k < extra.n; k++) {
-                  PT::combine(acc, loadGroupP(static_cast<const T*>(extra.p[k]), g, count, aligned), op);
+                  PT::combine(acc, loadGroup(static_cast<const T*>(extra.p[k]), g, count, aligned), op);
                 }
                 p[u] = PT::narrow(acc);
               }
@@ -222,44 +156,24 @@ pipelinedAllreduceKernel(CommArgs a, const T* in, T* out, size_t count, DevOp op
 namespace {
 template <typename T>
 const void* pipeFn(bool mc, int nranks) {
-  constexpr bool hot = std::is_same<T, float>::value || std::is_same<T, __half>::value || std::is_same<T, __nv_bfloat16>::value;
-  if constexpr (hot) {
-    if (mc) return reinterpret_cast<const void*>(pipelinedAllreduceKernel<T, true, 0>);
-    if (nranks == 2) return reinterpret_cast<const void*>(pipelinedAllreduceKernel<T, false, 2>);
-    if (nranks == 4) return reinterpret_cast<const void*>(pipelinedAllreduceKernel<T, false, 4>);
-    if (nranks == 8) return reinterpret_cast<const void*>(pipelinedAllreduceKernel<T, false, 8>);
+  if constexpr (isHotType<T>()) {
+    if (mc) return fn(pipelinedAllreduceKernel<T, true, 0>);
+    if (nranks == 2) return fn(pipelinedAllreduceKernel<T, false, 2>);
+    if (nranks == 4) return fn(pipelinedAllreduceKernel<T, false, 4>);
+    if (nranks == 8) return fn(pipelinedAllreduceKernel<T, false, 8>);
   }
-  return reinterpret_cast<const void*>(pipelinedAllreduceKernel<T, false, 0>);
-}
-
-const void* pipeKernelForImpl(DataType dt, bool mc, int nranks) {
-  switch (dt) {
-    case DataType::INT8: return pipeFn<int8_t>(false, nranks);
-    case DataType::UINT8: return pipeFn<uint8_t>(false, nranks);
-    case DataType::INT16: return pipeFn<int16_t>(false, nranks);
-    case DataType::INT32: return pipeFn<int32_t>(false, nranks);
-    case DataType::UINT32: return pipeFn<uint32_t>(false, nranks);
-    case DataType::INT64: return pipeFn<long long>(false, nranks);
-    case DataType::UINT64: return pipeFn<unsigned long long>(false, nranks);
-    case DataType::FLOAT32: return pipeFn<float>(mc, nranks);
-    case DataType::FLOAT64: return pipeFn<double>(false, nranks);
-    case DataType::FLOAT16: return pipeFn<__half>(mc, nranks);
-    case DataType::BFLOAT16: return pipeFn<__nv_bfloat16>(mc, nranks);
-  }
-  return nullptr;
+  return fn(pipelinedAllreduceKernel<T, false, 0>);
 }
 }  // namespace
 
-const void* pipelinedKernelFor(DataType dt, bool mc, int nranks) { return pipeKernelForImpl(dt, mc, nranks); }
+const void* pipelinedKernelFor(DataType dt, bool mc, int nranks) {
+  return dispatchType(dt, [&](auto t) { return pipeFn<decltype(t)>(mc, nranks); });
+}
 
 void preloadPipelineKernels() {
-  for (DataType dt : {DataType::INT8, DataType::UINT8, DataType::INT16, DataType::INT32, DataType::UINT32, DataType::INT64,
-                      DataType::UINT64, DataType::FLOAT32, DataType::FLOAT64, DataType::FLOAT16, DataType::BFLOAT16}) {
+  for (DataType dt : kAllDataTypes) {
     for (bool mc : {false, true}) {
-      for (int nr : {0, 2, 4, 8}) {
-        cudaFuncAttributes attr;
-        cudaFuncGetAttributes(&attr, pipeKernelForImpl(dt, mc, nr));
-      }
+      for (int nr : {0, 2, 4, 8}) touch(pipelinedKernelFor(dt, mc, nr));
     }
   }
   cudaGetLastError();
@@ -269,14 +183,13 @@ void launchPipelinedAllreduce(const CommArgs& a, const void* in, void* out, size
                               float scale, const PeerPtrs& stage, void* mcStage, int tileVecs, int exchangeThreads,
                               const LocalPtrs& extra, int blocks, cudaStream_t stream) {
   const bool mc = mcStage != nullptr && nvlsSupports(dt, op);
-  const void* k = pipeKernelForImpl(dt, mc, a.nranks);
   CommArgs ca = a;
   PeerPtrs st = stage;
   LocalPtrs ex = extra;
   char* mcp = mc ? static_cast<char*>(mcStage) : nullptr;
   DevOp dop = static_cast<DevOp>(op);
   void* args[] = {&ca, &in, &out, &count, &dop, &scale, &st, &mcp, &tileVecs, &exchangeThreads, &ex};
-  cudaLaunchKernel(k, dim3(static_cast<unsigned>(blocks)), dim3(kThreads), args, 0, stream);
+  launchKernel(pipelinedKernelFor(dt, mc, a.nranks), blocks, kThreads, args, stream);
 }
 
 }  // namespace cuda

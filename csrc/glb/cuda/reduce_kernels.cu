@@ -17,6 +17,7 @@
 
 #include "glb/common/utils.h"
 #include "glb/cuda/device_common.cuh"
+#include "glb/cuda/dispatch.cuh"
 #include "glb/cuda/kernels.h"
 
 namespace glb {
@@ -198,21 +199,18 @@ int gridFor(size_t items, int threads, int ctasPerSm = 4) {
   return static_cast<int>(want < 1 ? 1 : (want > cap ? cap : want));
 }
 
-template <typename F>
-void dispatchType(DataType dt, F&& f) {
-  switch (dt) {
-    case DataType::INT8: f(int8_t{}); break;
-    case DataType::UINT8: f(uint8_t{}); break;
-    case DataType::INT16: f(int16_t{}); break;
-    case DataType::INT32: f(int32_t{}); break;
-    case DataType::UINT32: f(uint32_t{}); break;
-    case DataType::INT64: f((long long){}); break;
-    case DataType::UINT64: f((unsigned long long){}); break;
-    case DataType::FLOAT32: f(float{}); break;
-    case DataType::FLOAT64: f(double{}); break;
-    case DataType::FLOAT16: f(__half{}); break;
-    case DataType::BFLOAT16: f(__nv_bfloat16{}); break;
+// The instantiation of the fused local allreduce for a launch shape (packs per thread and trip,
+// tiled or grid stride); an unroll other than 1 or 4 selects 2.
+template <typename T>
+const void* localAllreduceFn(int unroll, bool tiled) {
+  if (tiled) {
+    if (unroll == 4) return fn(localAllreduceManyKernel<T, 4, true>);
+    if (unroll == 1) return fn(localAllreduceManyKernel<T, 1, true>);
+    return fn(localAllreduceManyKernel<T, 2, true>);
   }
+  if (unroll == 4) return fn(localAllreduceManyKernel<T, 4, false>);
+  if (unroll == 1) return fn(localAllreduceManyKernel<T, 1, false>);
+  return fn(localAllreduceManyKernel<T, 2, false>);
 }
 
 bool aligned16(const void* p) { return reinterpret_cast<uintptr_t>(p) % 16 == 0; }
@@ -245,22 +243,14 @@ void launchLocalAllreduceMany(void* const* bufs, int n, size_t count, DataType d
     bp.p[i] = bufs[i];
     vectorOk = vectorOk && aligned16(bufs[i]);
   }
-  dispatchType(dt, [&](auto tag) {
-    using T = decltype(tag);
-    // Launch shape: measured on B200 (scripts/bench_local.py); GLB_LOCAL_SHAPE = "<ctas per SM>,<unroll>,<tiled>".
-    const LocalShape shape = localShape();
+  // Launch shape: measured on B200 (scripts/bench_local.py); GLB_LOCAL_SHAPE = "<ctas per SM>,<unroll>,<tiled>".
+  const LocalShape shape = localShape();
+  DevOp dop = static_cast<DevOp>(op);
+  void* args[] = {&bp, &n, &count, &dop, &scale, &vectorOk};
+  dispatchType(dt, [&](auto t) {
+    using T = decltype(t);
     const int grid = gridFor(count / PackTraits<T>::kElems / shape.unroll + 1, kLocalThreads, shape.ctasPerSm);
-    const DevOp dop = static_cast<DevOp>(op);
-    auto go = [&](auto kernel) { kernel<<<grid, kLocalThreads, 0, stream>>>(bp, n, count, dop, scale, vectorOk); };
-    if (shape.tiled) {
-      if (shape.unroll == 4) go(localAllreduceManyKernel<T, 4, true>);
-      else if (shape.unroll == 1) go(localAllreduceManyKernel<T, 1, true>);
-      else go(localAllreduceManyKernel<T, 2, true>);
-    } else {
-      if (shape.unroll == 4) go(localAllreduceManyKernel<T, 4, false>);
-      else if (shape.unroll == 1) go(localAllreduceManyKernel<T, 1, false>);
-      else go(localAllreduceManyKernel<T, 2, false>);
-    }
+    launchKernel(localAllreduceFn<T>(shape.unroll, shape.tiled), grid, kLocalThreads, args, stream);
   });
 }
 
@@ -309,27 +299,19 @@ void setLocalAllreduceShape(int ctasPerSm, int unroll, bool tiled) {
 }
 
 void preloadLocalKernels() {
-  auto touch = [](const void* k) {
-    cudaFuncAttributes attr;
-    cudaFuncGetAttributes(&attr, k);
-  };
-  for (DataType dt : {DataType::INT8, DataType::UINT8, DataType::INT16, DataType::INT32, DataType::UINT32, DataType::INT64,
-                      DataType::UINT64, DataType::FLOAT32, DataType::FLOAT64, DataType::FLOAT16, DataType::BFLOAT16}) {
-    dispatchType(dt, [&](auto tag) {
-      using T = decltype(tag);
-      touch(reinterpret_cast<const void*>(localReduceManyKernel<T>));
-      touch(reinterpret_cast<const void*>(localAllreduceManyKernel<T, 1, false>));
-      touch(reinterpret_cast<const void*>(localAllreduceManyKernel<T, 2, false>));
-      touch(reinterpret_cast<const void*>(localAllreduceManyKernel<T, 4, false>));
-      touch(reinterpret_cast<const void*>(localAllreduceManyKernel<T, 1, true>));
-      touch(reinterpret_cast<const void*>(localAllreduceManyKernel<T, 2, true>));
-      touch(reinterpret_cast<const void*>(localAllreduceManyKernel<T, 4, true>));
-      touch(reinterpret_cast<const void*>(verifyKernel<T>));
-      touch(reinterpret_cast<const void*>(fillKernel<T>));
+  for (DataType dt : kAllDataTypes) {
+    dispatchType(dt, [](auto t) {
+      using T = decltype(t);
+      touch(fn(localReduceManyKernel<T>));
+      touch(fn(verifyKernel<T>));
+      touch(fn(fillKernel<T>));
+      for (int unroll : {1, 2, 4}) {
+        for (bool tiled : {false, true}) touch(localAllreduceFn<T>(unroll, tiled));
+      }
     });
   }
-  touch(reinterpret_cast<const void*>(localBroadcastKernel));
-  touch(reinterpret_cast<const void*>(spinKernel));
+  touch(fn(localBroadcastKernel));
+  touch(fn(spinKernel));
   cudaGetLastError();
 }
 

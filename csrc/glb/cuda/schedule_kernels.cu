@@ -1,5 +1,6 @@
 // Generic step-table executor for the literal allreduce schedules (see schedules.h).
 #include "glb/cuda/device_common.cuh"
+#include "glb/cuda/dispatch.cuh"
 #include "glb/cuda/schedules.h"
 
 namespace glb {
@@ -102,7 +103,7 @@ scheduleKernel(CommArgs a, PeerPtrs bufs, PeerPtrs stage, const SchedStep* __res
       }
       for (size_t i = firstOwned(tailBegin); i < tailEnd; i += nthreads) {
         T acc = local[i];
-        for (int p = 0; p < st.npeers; p++) acc = PT::combineOne(acc, static_cast<const T*>(srcs.p[st.peers[p]])[i], op);
+        for (int p = 0; p < st.npeers; p++) acc = combineOne<T>(acc, static_cast<const T*>(srcs.p[st.peers[p]])[i], op);
         local[i] = acc;
       }
     }
@@ -118,53 +119,30 @@ scheduleKernel(CommArgs a, PeerPtrs bufs, PeerPtrs stage, const SchedStep* __res
         PT::scale(acc, scale);
         st128(lbase + v * 16, PT::narrow(acc));
       }
-      for (size_t i = nvec * PT::kElems + tid; i < count; i += nthreads) local[i] = PT::scaleOne(local[i], scale);
+      for (size_t i = nvec * PT::kElems + tid; i < count; i += nthreads) local[i] = scaleOne<T>(local[i], scale);
     }
   }
   retire(a, static_cast<uint32_t>(nbarriers), 0);
 }
 
+namespace {
+const void* scheduleKernelFor(DataType dt) {
+  return dispatchType(dt, [](auto t) { return fn(scheduleKernel<decltype(t)>); });
+}
+}  // namespace
+
 void launchSchedule(const CommArgs& a, const PeerPtrs& bufs, const PeerPtrs& stage, const SchedStep* table,
                     int nsteps, int nbarriers, DataType dt, ReduceOp op, float scale, size_t count, bool vectorOk,
                     int blocks, cudaStream_t stream) {
-  const DevOp dop = static_cast<DevOp>(op);
-#define GLB_CASE(E, T)                                                                                          \
-  case DataType::E:                                                                                             \
-    scheduleKernel<T><<<blocks, kThreads, 0, stream>>>(a, bufs, stage, table, nsteps, nbarriers, dop, scale, count, vectorOk); \
-    break;
-  switch (dt) {
-    GLB_CASE(INT8, int8_t)
-    GLB_CASE(UINT8, uint8_t)
-    GLB_CASE(INT16, int16_t)
-    GLB_CASE(INT32, int32_t)
-    GLB_CASE(UINT32, uint32_t)
-    GLB_CASE(INT64, long long)
-    GLB_CASE(UINT64, unsigned long long)
-    GLB_CASE(FLOAT32, float)
-    GLB_CASE(FLOAT64, double)
-    GLB_CASE(FLOAT16, __half)
-    GLB_CASE(BFLOAT16, __nv_bfloat16)
-  }
-#undef GLB_CASE
+  CommArgs ca = a;
+  PeerPtrs pb = bufs, ps = stage;
+  DevOp dop = static_cast<DevOp>(op);
+  void* args[] = {&ca, &pb, &ps, &table, &nsteps, &nbarriers, &dop, &scale, &count, &vectorOk};
+  launchKernel(scheduleKernelFor(dt), blocks, kThreads, args, stream);
 }
 
-
 void preloadScheduleKernels() {
-  auto touch = [](const void* k) {
-    cudaFuncAttributes attr;
-    cudaFuncGetAttributes(&attr, k);
-  };
-  touch(reinterpret_cast<const void*>(scheduleKernel<int8_t>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<uint8_t>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<int16_t>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<int32_t>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<uint32_t>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<long long>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<unsigned long long>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<float>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<double>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<__half>));
-  touch(reinterpret_cast<const void*>(scheduleKernel<__nv_bfloat16>));
+  for (DataType dt : kAllDataTypes) touch(scheduleKernelFor(dt));
   cudaGetLastError();
 }
 
