@@ -454,6 +454,73 @@ void launchGatherPush(const CommArgs& a, const void* in, const PeerPtrs& outs, v
                                                     va, onlyDst, vec);
 }
 
+// ---- allgather(v) with a dtype conversion --------------------------------------------------
+// Same barriers and grid rule as gatherPushKernel; offsets and lengths are in ELEMENTS. Rank r
+// reads its block once as TI, converts it once (round to nearest even when narrowing, exact
+// when widening) and stores it at element offset off[r] of every rank's TO output, peers
+// rotated. Items of 8 elements while `in` and my output byte offset are 16-byte aligned.
+template <typename TI, typename TO>
+__global__ void __launch_bounds__(kThreads, 2)
+gatherPushCastKernel(CommArgs a, const TI* __restrict__ in, PeerPtrs outs, VArgs va, bool vec) {
+  using II = Item8<TI>;
+  using OI = Item8<TO>;
+  const uint32_t e = loadEpoch(a);
+  const size_t tid = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const size_t nthreads = static_cast<size_t>(gridDim.x) * blockDim.x;
+  const int P = a.nranks;
+  if (!blockBarrier<false>(a, e + 1)) {
+    retire(a, 2, 0);
+    return;
+  }
+  const size_t off = va.off[a.rank], len = va.len[a.rank];
+  const size_t outByte = off * sizeof(TO);
+  const bool v16 = vec && reinterpret_cast<uintptr_t>(in) % 16 == 0 && outByte % 16 == 0;
+  const size_t nitems = v16 ? len / 8 : 0;
+  constexpr int U = sizeof(TI) == 4 ? 2 : 4;  // 64 bytes of input in flight per thread
+  for (size_t i0 = tid; i0 < nitems; i0 += nthreads * U) {
+    float v[U][8];
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+      const size_t it = i0 + u * nthreads;
+      if (it < nitems) II::load(reinterpret_cast<const char*>(in) + it * II::kBytes, v[u]);
+    }
+    for (int i = 0; i < P; i++) {
+      char* dst = static_cast<char*>(outs.p[(a.rank + i) % P]) + outByte;
+#pragma unroll
+      for (int u = 0; u < U; u++) {
+        const size_t it = i0 + u * nthreads;
+        if (it < nitems) OI::store(dst + it * OI::kBytes, v[u]);
+      }
+    }
+  }
+  for (size_t i = nitems * 8 + tid; i < len; i += nthreads) {
+    const TO o = fromAcc<TO, float>(toAcc<TI>(in[i]));
+    for (int r = 0; r < P; r++) static_cast<TO*>(outs.p[(a.rank + r) % P])[off + i] = o;
+  }
+  blockBarrier(a, e + 2);
+  retire(a, 2, 0);
+}
+
+const void* gatherPushCastKernelFor(DataType in, DataType out) {
+  return dispatchCast(in, out, [](auto ti, auto to) { return fn(gatherPushCastKernel<decltype(ti), decltype(to)>); });
+}
+
+void launchGatherPushCast(const CommArgs& a, const void* in, const PeerPtrs& outs, const size_t* elemOff,
+                          const size_t* elemLen, DataType dt, DataType outDt, bool vec, int blocks,
+                          cudaStream_t stream) {
+  const void* k = gatherPushCastKernelFor(dt, outDt);
+  if (k == nullptr) return;
+  VArgs va;
+  for (int i = 0; i < kMaxRanks; i++) {
+    va.off[i] = i < a.nranks ? elemOff[i] : 0;
+    va.len[i] = i < a.nranks ? elemLen[i] : 0;
+  }
+  CommArgs ca = a;
+  PeerPtrs po = outs;
+  void* args[] = {&ca, &in, &po, &va, &vec};
+  launchKernel(k, blocks, kThreads, args, stream);
+}
+
 // ---- alltoall(v) / scatter: push chunk j of my input into slot (me) of rank j's output -------
 // sendOff/sendLen index my input per destination; recvOff[r] (same on all ranks by
 // symmetry of the exchange tables) is where MY chunk lands in rank r's output.
@@ -654,6 +721,135 @@ void launchReducePull(const CommArgs& a, const PeerPtrs& ins, void* mcIn, void* 
   launchKernel(reducePullKernelPtr(dt, a.nranks), blocks, kThreads, args, stream);
 }
 
+// ---- reduce_scatter with a dtype conversion --------------------------------------------------
+// Same barriers, CTA pairing and share tables as reducePullKernel. Rank r pulls its share of
+// every peer's TI input in rank-rotated order, accumulates in fp32, applies `scale` to the
+// accumulator, rounds once to TO and stores to its local `out`. Items of 8 elements while my
+// input byte offset and `out` are 16-byte aligned; the rank-count specialisations load every
+// peer's item before reducing any (UNROLL items per thread), as reducePullKernel does. It never uses
+// multimem.ld_reduce: the switch returns the input dtype, so a 16-bit input would be rounded
+// to 16 bits before the fp32 result is formed.
+template <typename TI, typename TO, int NR, int UNROLL>
+__global__ void __launch_bounds__(kThreads, 1)
+reducePullCastKernel(CommArgs a, PeerPtrs ins, TO* __restrict__ out, EArgs ea, DevOp op, float scale, bool vec) {
+  using II = Item8<TI>;
+  using OI = Item8<TO>;
+  constexpr int kPk = II::kPacks;
+  const uint32_t e = loadEpoch(a);
+  const size_t tid = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const size_t nthreads = static_cast<size_t>(gridDim.x) * blockDim.x;
+  const int P = NR > 0 ? NR : a.nranks;
+  if (!blockBarrier<false>(a, e + 1)) {
+    retire(a, 2, 0);
+    return;
+  }
+  const size_t off = ea.off[a.rank], len = ea.len[a.rank];
+  const size_t byteOff = off * sizeof(TI);
+  const bool v16 = vec && byteOff % 16 == 0 && reinterpret_cast<uintptr_t>(out) % 16 == 0;
+  const size_t nitems = v16 ? len / 8 : 0;
+  if constexpr (NR > 0) {
+    const char* peer[NR];
+#pragma unroll
+    for (int i = 0; i < NR; i++) peer[i] = static_cast<const char*>(ins.p[(a.rank + i) % NR]) + byteOff;
+    for (size_t i0 = tid; i0 < nitems; i0 += nthreads * UNROLL) {
+      Pack16 p[UNROLL][NR][kPk];
+#pragma unroll
+      for (int u = 0; u < UNROLL; u++) {
+        const size_t it = i0 + static_cast<size_t>(u) * nthreads;
+        if (it < nitems) {
+#pragma unroll
+          for (int i = 0; i < NR; i++) {
+#pragma unroll
+            for (int k = 0; k < kPk; k++) p[u][i][k] = ld128_stream(peer[i] + it * II::kBytes + k * 16);
+          }
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < UNROLL; u++) {
+        const size_t it = i0 + static_cast<size_t>(u) * nthreads;
+        if (it < nitems) {
+          float acc[8];
+          II::widen(p[u][0], acc);
+#pragma unroll
+          for (int i = 1; i < NR; i++) {
+            float x[8];
+            II::widen(p[u][i], x);
+#pragma unroll
+            for (int k = 0; k < 8; k++) acc[k] = applyOp<float>(acc[k], x[k], op);
+          }
+          if (scale != 1.0f) {
+#pragma unroll
+            for (int k = 0; k < 8; k++) acc[k] *= scale;
+          }
+          OI::template store<false>(reinterpret_cast<char*>(out) + it * OI::kBytes, acc);
+        }
+      }
+    }
+  } else {
+    // Any rank count: one peer's item at a time.
+    for (size_t it = tid; it < nitems; it += nthreads) {
+      float acc[8];
+      II::load(static_cast<const char*>(ins.p[a.rank]) + byteOff + it * II::kBytes, acc);
+      for (int i = 1; i < P; i++) {
+        float x[8];
+        II::load(static_cast<const char*>(ins.p[(a.rank + i) % P]) + byteOff + it * II::kBytes, x);
+#pragma unroll
+        for (int k = 0; k < 8; k++) acc[k] = applyOp<float>(acc[k], x[k], op);
+      }
+      if (scale != 1.0f) {
+#pragma unroll
+        for (int k = 0; k < 8; k++) acc[k] *= scale;
+      }
+      OI::template store<false>(reinterpret_cast<char*>(out) + it * OI::kBytes, acc);
+    }
+  }
+  for (size_t i = nitems * 8 + tid; i < len; i += nthreads) {
+    float acc = toAcc<TI>(static_cast<const TI*>(ins.p[a.rank])[off + i]);
+    for (int r = 1; r < P; r++) {
+      acc = applyOp<float>(acc, toAcc<TI>(static_cast<const TI*>(ins.p[(a.rank + r) % P])[off + i]), op);
+    }
+    if (scale != 1.0f) acc = scaleAcc(acc, scale);
+    out[i] = fromAcc<TO, float>(acc);
+  }
+  blockBarrier(a, e + 2);
+  retire(a, 2, 0);
+}
+
+namespace {
+// The instantiation for (TI, TO, P): rank-count specialisations with the unroll of
+// reducePullFn for 16-bit inputs, half of it for f32 inputs (twice the bytes per item), so
+// both keep the same bytes in flight per thread as the same-dtype pull kernel.
+template <typename TI, typename TO>
+const void* reducePullCastFn(int P) {
+  constexpr int W = sizeof(TI) == 4 ? 2 : 1;
+  if (P == 2) return fn(reducePullCastKernel<TI, TO, 2, 4 / W>);
+  if (P == 4) return fn(reducePullCastKernel<TI, TO, 4, 2 / W>);
+  if (P == 8) return fn(reducePullCastKernel<TI, TO, 8, 2 / W>);
+  return fn(reducePullCastKernel<TI, TO, 0, 1>);
+}
+}  // namespace
+
+const void* reducePullCastKernelFor(DataType in, DataType out, int nranks) {
+  return dispatchCast(in, out, [&](auto ti, auto to) { return reducePullCastFn<decltype(ti), decltype(to)>(nranks); });
+}
+
+void launchReducePullCast(const CommArgs& a, const PeerPtrs& ins, void* out, const size_t* elemOff,
+                          const size_t* elemLen, DataType dt, DataType outDt, ReduceOp op, float scale, bool vec,
+                          int blocks, cudaStream_t stream) {
+  const void* k = reducePullCastKernelFor(dt, outDt, a.nranks);
+  if (k == nullptr) return;
+  EArgs ea;
+  for (int i = 0; i < kMaxRanks; i++) {
+    ea.off[i] = i < a.nranks ? elemOff[i] : 0;
+    ea.len[i] = i < a.nranks ? elemLen[i] : 0;
+  }
+  CommArgs ca = a;
+  PeerPtrs pi = ins;
+  DevOp dop = static_cast<DevOp>(op);
+  void* args[] = {&ca, &pi, &out, &ea, &dop, &scale, &vec};
+  launchKernel(k, blocks, kThreads, args, stream);
+}
+
 
 // ---- small allgather / alltoall without a barrier: flag-in-data lines -------------------------
 // Same protocol and pool region as llAllreduceKernel (every rank hears from every peer in a
@@ -746,6 +942,10 @@ void preloadCollectiveKernels() {
   touch(fn(llExchangeKernel));
   for (DataType dt : kAllDataTypes) {
     for (int P : {0, 2, 4, 8}) touch(reducePullKernelPtr(dt, P));
+    for (DataType outDt : kAllDataTypes) {
+      touch(gatherPushCastKernelFor(dt, outDt));
+      for (int P : {0, 2, 4, 8}) touch(reducePullCastKernelFor(dt, outDt, P));
+    }
   }
   cudaGetLastError();
 }

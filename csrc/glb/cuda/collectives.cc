@@ -206,6 +206,20 @@ void runLL(PeerContext& pc, const void* in, void* out, size_t count, DataType dt
                     extra, blocks, threads, stream);
 }
 
+// Single rank with a dtype conversion: the LL kernel degenerates to a local scale and
+// convert; it runs in pieces the LL region accepts.
+void localCast(PeerContext& pc, const void* in, void* out, size_t count, DataType dt, DataType outDt, ReduceOp op,
+               float scale, cudaStream_t stream, const char* what) {
+  const size_t piece = pc.llMaxBytes() / elementSize(dt);
+  pc.checkHealth();
+  for (size_t done = 0; done < count; done += piece) {
+    const size_t n = std::min(piece, count - done);
+    runLL(pc, static_cast<const char*>(in) + done * elementSize(dt), static_cast<char*>(out) + done * elementSize(outDt),
+          n, dt, outDt, op, scale, LocalPtrs(), 0, stream);
+    checkLaunch(what);
+  }
+}
+
 void runOneShot(PeerContext& pc, const void* in, void* out, size_t count, DataType dt, ReduceOp op, float scale,
                 const LocalPtrs& extra, int blocksHint, cudaStream_t stream) {
   const auto l = layoutOf(pc);
@@ -405,16 +419,8 @@ void allreduceCast(PeerContext& pc, const PeerBuffer& in, size_t inOffset, const
   const float scale = scaleOf(ep, DataType::FLOAT32);
   DeviceGuard g(pc.device);
   if (pc.size == 1 && !envFlag("CUDA_FORCE_KERNELS", false)) {
-    // Degenerate: convert (and scale) locally, in pieces the LL kernel accepts.
-    const size_t piece = pc.llMaxBytes() / elementSize(dt);
-    pc.checkHealth();
-    for (size_t done = 0; done < count; done += piece) {
-      const size_t n = std::min(piece, count - done);
-      runLL(pc, static_cast<const char*>(in.local) + inOffset + done * elementSize(dt),
-            static_cast<char*>(out.local) + outOffset + done * elementSize(outDt), n, dt, outDt, op, scale, LocalPtrs(), 0,
-            stream);
-      checkLaunch("allreduceCast(local)");
-    }
+    localCast(pc, static_cast<const char*>(in.local) + inOffset, static_cast<char*>(out.local) + outOffset, count, dt,
+              outDt, op, scale, stream, "allreduceCast(local)");
     return;
   }
   const bool vec = in.vectorOk && out.vectorOk && inOffset % 32 == 0 && outOffset % 32 == 0;
@@ -640,6 +646,70 @@ void allgatherv(PeerContext& pc, const void* in, void* out, const std::vector<si
   auto st = stagedBulk(pc, off.back(), "allgather");
   gatherCommon(pc, in, st.ptrs, nullptr, true, bytesPerRank, -1, stream);
   if (off.back() > 0) GLB_CUDA_CHECK(cudaMemcpyAsync(out, st.mine, off.back(), cudaMemcpyDeviceToDevice, stream));
+}
+
+namespace {
+std::vector<size_t> bytesOf(const std::vector<size_t>& counts, DataType dt) {
+  std::vector<size_t> b(counts);
+  for (size_t& x : b) x *= elementSize(dt);
+  return b;
+}
+
+void checkCast(DataType in, DataType out, const char* what) {
+  GLB_ENFORCE(castSupported(in, out), what, ": supported conversions are f32 -> f16 / bf16 and f16 / bf16 -> f32");
+}
+
+// No LL variant and no multicast: the push kernel with a conversion, grid from the largest
+// block's OUTPUT bytes (the "allgather" table entry), identical on every rank.
+void gatherCastCommon(PeerContext& pc, const void* in, DataType inDt, const PeerPtrs& outs, bool vecOut,
+                      const std::vector<size_t>& counts, DataType outDt, cudaStream_t stream) {
+  GLB_TRACE_RANGE("glb::cuda::allgatherCast");
+  auto off = prefix(counts);
+  const size_t largest = *std::max_element(counts.begin(), counts.end());
+  const bool vec = vecOut && reinterpret_cast<uintptr_t>(in) % 16 == 0;
+  const int blocks = bwBlocks(pc, "allgather", gatherPushCastKernelFor(inDt, outDt), largest * elementSize(outDt));
+  prologue(pc, stream);
+  launchGatherPushCast(pc.comm(), in, outs, off.data(), counts.data(), inDt, outDt, vec, blocks, stream);
+  finish(pc, stream, "allgatherCast");
+}
+}  // namespace
+
+void allgathervCast(PeerContext& pc, const void* in, DataType inDt, const PeerBuffer& out, size_t outOffset,
+                    const std::vector<size_t>& counts, DataType outDt, cudaStream_t stream) {
+  if (inDt == outDt) {
+    allgatherv(pc, in, out, outOffset, bytesOf(counts, inDt), stream);
+    return;
+  }
+  checkCast(inDt, outDt, "allgatherCast");
+  GLB_ENFORCE_EQ(static_cast<int>(counts.size()), pc.size, "need one element count per rank");
+  DeviceGuard g(pc.device);
+  auto off = prefix(counts);
+  GLB_ENFORCE_LE(outOffset + off.back() * elementSize(outDt), out.bytes, "allgather output exceeds the registered buffer");
+  char* dst = static_cast<char*>(out.local) + outOffset;
+  if (pc.size == 1) {
+    localCast(pc, in, dst, counts[0], inDt, outDt, ReduceOp::SUM, 1.0f, stream, "allgatherCast(local)");
+    return;
+  }
+  gatherCastCommon(pc, in, inDt, out.ptrsAt(outOffset), out.vectorOk && outOffset % 16 == 0, counts, outDt, stream);
+}
+
+void allgathervCast(PeerContext& pc, const void* in, DataType inDt, void* out, const std::vector<size_t>& counts,
+                    DataType outDt, cudaStream_t stream) {
+  if (inDt == outDt) {
+    allgatherv(pc, in, out, bytesOf(counts, inDt), stream);
+    return;
+  }
+  checkCast(inDt, outDt, "allgatherCast");
+  GLB_ENFORCE_EQ(static_cast<int>(counts.size()), pc.size, "need one element count per rank");
+  DeviceGuard g(pc.device);
+  if (pc.size == 1) {
+    localCast(pc, in, out, counts[0], inDt, outDt, ReduceOp::SUM, 1.0f, stream, "allgatherCast(local)");
+    return;
+  }
+  const size_t outBytes = prefix(counts).back() * elementSize(outDt);
+  auto st = stagedBulk(pc, outBytes, "allgather");
+  gatherCastCommon(pc, in, inDt, st.ptrs, true, counts, outDt, stream);
+  if (outBytes > 0) GLB_CUDA_CHECK(cudaMemcpyAsync(out, st.mine, outBytes, cudaMemcpyDeviceToDevice, stream));
 }
 
 void gatherv(PeerContext& pc, const void* in, const PeerBuffer& out, size_t outOffset,
@@ -878,6 +948,78 @@ void reduce_scatter(PeerContext& pc, const void* in, void* out, const std::vecto
   auto st = stagedBulk(pc, off.back() * es, "reduce_scatter");
   if (off.back() > 0) GLB_CUDA_CHECK(cudaMemcpyAsync(st.mine, in, off.back() * es, cudaMemcpyDeviceToDevice, stream));
   reducePullCommon(pc, st.ptrs, st.mc, true, out, counts, dt, op, scale, stream);
+}
+
+namespace {
+// The pull kernel with a conversion. Grid from the "reduce_scatter" table entry keyed by the
+// largest share's INPUT bytes, as reducePullCommon sizes it; the kernel reads peers directly,
+// so the entry for registered buffers applies whether or not the input has a multicast alias.
+void reducePullCastCommon(PeerContext& pc, const PeerPtrs& ins, bool vecIn, void* out, const std::vector<size_t>& counts,
+                          DataType dt, DataType outDt, ReduceOp op, float scale, cudaStream_t stream) {
+  GLB_TRACE_RANGE("glb::cuda::reduceScatterCast");
+  auto off = prefix(counts);
+  const size_t inBytes = *std::max_element(counts.begin(), counts.end()) * elementSize(dt);
+  int cap = tuning().maxBlocks;
+  if (const TuneEntry* e = TuningTable::get().lookup("reduce_scatter", pc.size, BufKind::REGISTERED, inBytes)) {
+    if (e->blocks > 0) cap = e->blocks;
+  }
+  const int blocks =
+      std::min(blocksFor(pc, inBytes / 16, 1, cap), pc.coResidentBlocks(reducePullCastKernelFor(dt, outDt, pc.size)));
+  prologue(pc, stream);
+  launchReducePullCast(pc.comm(), ins, out, off.data(), counts.data(), dt, outDt, op, scale, vecIn, blocks, stream);
+  finish(pc, stream, "reduceScatterCast");
+}
+
+// Checks shared by both reduceScatterCast overloads; returns the scale as the kernels take it.
+float reduceScatterCastArgs(PeerContext& pc, const std::vector<size_t>& counts, DataType dt, DataType outDt,
+                            ReduceOp op, double scaleD) {
+  checkCast(dt, outDt, "reduceScatterCast");
+  GLB_ENFORCE(op != ReduceOp::CUSTOM, "custom reductions run on the host path only");
+  GLB_ENFORCE_EQ(static_cast<int>(counts.size()), pc.size, "need one element count per rank");
+  Epilogue ep;
+  ep.scale = scaleD;
+  return scaleOf(ep, DataType::FLOAT32);
+}
+}  // namespace
+
+void reduceScatterCast(PeerContext& pc, const PeerBuffer& in, size_t inOffset, void* out,
+                       const std::vector<size_t>& counts, DataType dt, DataType outDt, ReduceOp op,
+                       cudaStream_t stream, double scaleD) {
+  if (dt == outDt) {
+    reduce_scatter(pc, in, inOffset, out, counts, dt, op, stream, scaleD);
+    return;
+  }
+  const float scale = reduceScatterCastArgs(pc, counts, dt, outDt, op, scaleD);
+  DeviceGuard g(pc.device);
+  auto off = prefix(counts);
+  GLB_ENFORCE_LE(inOffset + off.back() * elementSize(dt), in.bytes, "reduce_scatter input exceeds the registered buffer");
+  const char* src = static_cast<const char*>(in.local) + inOffset;
+  // A single rank converts locally in every overload, like reduce_scatter / allgatherv, which
+  // copy locally whatever GLB_CUDA_FORCE_KERNELS says.
+  if (pc.size == 1) {
+    localCast(pc, src, out, counts[0], dt, outDt, op, scale, stream, "reduceScatterCast(local)");
+    return;
+  }
+  reducePullCastCommon(pc, in.ptrsAt(inOffset), in.vectorOk && inOffset % 16 == 0, out, counts, dt, outDt, op, scale,
+                       stream);
+}
+
+void reduceScatterCast(PeerContext& pc, const void* in, void* out, const std::vector<size_t>& counts, DataType dt,
+                       DataType outDt, ReduceOp op, cudaStream_t stream, double scaleD) {
+  if (dt == outDt) {
+    reduce_scatter(pc, in, out, counts, dt, op, stream, scaleD);
+    return;
+  }
+  const float scale = reduceScatterCastArgs(pc, counts, dt, outDt, op, scaleD);
+  DeviceGuard g(pc.device);
+  if (pc.size == 1) {
+    localCast(pc, in, out, counts[0], dt, outDt, op, scale, stream, "reduceScatterCast(local)");
+    return;
+  }
+  const size_t inBytes = prefix(counts).back() * elementSize(dt);
+  auto st = stagedBulk(pc, inBytes, "reduce_scatter");
+  if (inBytes > 0) GLB_CUDA_CHECK(cudaMemcpyAsync(st.mine, in, inBytes, cudaMemcpyDeviceToDevice, stream));
+  reducePullCastCommon(pc, st.ptrs, true, out, counts, dt, outDt, op, scale, stream);
 }
 
 void reduce(PeerContext& pc, const PeerBuffer& in, size_t inOffset, const PeerBuffer& out, size_t outOffset,

@@ -123,6 +123,14 @@ void allgatherv(PeerContext& pc, const void* in, const PeerBuffer& out, size_t o
                 const std::vector<size_t>& bytesPerRank, cudaStream_t stream);
 void allgatherv(PeerContext& pc, const void* in, void* out, const std::vector<size_t>& bytesPerRank,
                 cudaStream_t stream);
+// allgatherv with a dtype conversion (f32 -> f16 / bf16 rounds to nearest even, f16 / bf16 ->
+// f32 is exact): rank r's `in` (counts[r] ELEMENTS of inDt) lands, converted to outDt, at the
+// prefix-sum element offset of every out. Each block is read and converted once. Same dtypes:
+// allgatherv.
+void allgathervCast(PeerContext& pc, const void* in, DataType inDt, const PeerBuffer& out, size_t outOffset,
+                    const std::vector<size_t>& counts, DataType outDt, cudaStream_t stream);
+void allgathervCast(PeerContext& pc, const void* in, DataType inDt, void* out, const std::vector<size_t>& counts,
+                    DataType outDt, cudaStream_t stream);
 // Only `root` receives.
 void gatherv(PeerContext& pc, const void* in, const PeerBuffer& out, size_t outOffset,
              const std::vector<size_t>& bytesPerRank, int root, cudaStream_t stream);
@@ -151,6 +159,14 @@ void reduce_scatter(PeerContext& pc, const PeerBuffer& in, size_t inOffset, void
                     double scale = 1.0);
 void reduce_scatter(PeerContext& pc, const void* in, void* out, const std::vector<size_t>& counts, DataType dt,
                     ReduceOp op, cudaStream_t stream, double scale = 1.0);
+// reduce_scatter of `dt` inputs into an `outDt` output (f32 <-> f16 / bf16): fp32 accumulation,
+// `scale` on the accumulator, one rounding to outDt. One barrier kernel at every size (no LL
+// variant) and never multicast. Same dtypes: reduce_scatter.
+void reduceScatterCast(PeerContext& pc, const PeerBuffer& in, size_t inOffset, void* out,
+                       const std::vector<size_t>& counts, DataType dt, DataType outDt, ReduceOp op,
+                       cudaStream_t stream, double scale = 1.0);
+void reduceScatterCast(PeerContext& pc, const void* in, void* out, const std::vector<size_t>& counts, DataType dt,
+                       DataType outDt, ReduceOp op, cudaStream_t stream, double scale = 1.0);
 // Reduction of every rank's `in` delivered to root's `out` (both registered).
 void reduce(PeerContext& pc, const PeerBuffer& in, size_t inOffset, const PeerBuffer& out, size_t outOffset,
             size_t count, DataType dt, ReduceOp op, int root, cudaStream_t stream);

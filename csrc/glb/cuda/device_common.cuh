@@ -401,25 +401,47 @@ struct PackTraits<__nv_bfloat16> {
 // ---- mixed-precision items (cast epilogue) --------------------------------------------
 // Eight consecutive elements of T as fp32 lanes: 2 x 16 B for float, 1 x 16 B for the
 // 16-bit types. Used by the kernels whose output dtype differs from the input dtype
-// (fp32 accumulate -> bf16/fp16 store, or 16-bit inputs -> fp32 result).
+// (fp32 accumulate -> bf16/fp16 store, or 16-bit inputs -> fp32 result). `widen` turns
+// kPacks raw packs into the lanes, for kernels that issue all their loads before using them.
+// `store<false>` stores with plain st.global (no L1::no_allocate) for a local output that is
+// read again soon, as the same-dtype reduce_scatter does.
 template <typename T>  // __half, __nv_bfloat16
 struct Item8 {
   static constexpr int kBytes = 16;
+  static constexpr int kPacks = 1;
+  __device__ static void widen(const Pack16 (&p)[kPacks], float (&v)[8]) {
+    const auto a = PackTraits<T>::widen(p[0]);
+#pragma unroll
+    for (int i = 0; i < 8; i++) v[i] = a.v[i];
+  }
   __device__ static void load(const void* p, float (&v)[8]) {
     const auto a = PackTraits<T>::widen(ld128_stream(p));
 #pragma unroll
     for (int i = 0; i < 8; i++) v[i] = a.v[i];
   }
+  template <bool kStream = true>
   __device__ static void store(void* p, const float (&v)[8]) {
     typename PackTraits<T>::AccPack a;
 #pragma unroll
     for (int i = 0; i < 8; i++) a.v[i] = v[i];
-    st128_stream(p, PackTraits<T>::narrow(a));
+    if constexpr (kStream) {
+      st128_stream(p, PackTraits<T>::narrow(a));
+    } else {
+      st128(p, PackTraits<T>::narrow(a));
+    }
   }
 };
 template <>
 struct Item8<float> {
   static constexpr int kBytes = 32;
+  static constexpr int kPacks = 2;
+  __device__ static void widen(const Pack16 (&p)[kPacks], float (&v)[8]) {
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      v[i] = __uint_as_float(p[0].w[i]);
+      v[4 + i] = __uint_as_float(p[1].w[i]);
+    }
+  }
   __device__ static void load(const void* p, float (&v)[8]) {
     const Pack16 a = ld128_stream(p), b = ld128_stream(static_cast<const char*>(p) + 16);
 #pragma unroll
@@ -428,6 +450,7 @@ struct Item8<float> {
       v[4 + i] = __uint_as_float(b.w[i]);
     }
   }
+  template <bool kStream = true>
   __device__ static void store(void* p, const float (&v)[8]) {
     Pack16 a, b;
 #pragma unroll
@@ -435,8 +458,13 @@ struct Item8<float> {
       a.w[i] = __float_as_uint(v[i]);
       b.w[i] = __float_as_uint(v[4 + i]);
     }
-    st128_stream(p, a);
-    st128_stream(static_cast<char*>(p) + 16, b);
+    if constexpr (kStream) {
+      st128_stream(p, a);
+      st128_stream(static_cast<char*>(p) + 16, b);
+    } else {
+      st128(p, a);
+      st128(static_cast<char*>(p) + 16, b);
+    }
   }
 };
 

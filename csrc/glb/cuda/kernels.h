@@ -70,12 +70,23 @@ void launchAlltoallPush(const CommArgs& a, const void* in, const PeerPtrs& outs,
 void launchReducePull(const CommArgs& a, const PeerPtrs& ins, void* mcIn, void* out, const size_t* elemOff,
                       const size_t* elemLen, DataType dt, ReduceOp op, float scale, bool vec, bool useMc, int blocks,
                       cudaStream_t stream);
+// The same two collectives with a dtype conversion (one of castSupported's pairs, dt != outDt).
+// Offsets and lengths are in elements. reduce_scatter: fp32 accumulation, scale, one rounding
+// to outDt, never multicast. allgather: each block converted once, no scale.
+void launchReducePullCast(const CommArgs& a, const PeerPtrs& ins, void* out, const size_t* elemOff,
+                          const size_t* elemLen, DataType dt, DataType outDt, ReduceOp op, float scale, bool vec,
+                          int blocks, cudaStream_t stream);
+void launchGatherPushCast(const CommArgs& a, const void* in, const PeerPtrs& outs, const size_t* elemOff,
+                          const size_t* elemLen, DataType dt, DataType outDt, bool vec, int blocks,
+                          cudaStream_t stream);
 // Entry points, for occupancy queries (every CTA of a collective kernel must be resident).
 const void* broadcastKernelPtr();
 const void* gatherPushKernelPtr();
 const void* gatherBulkKernelPtr();
 const void* alltoallPushKernelPtr();
 const void* reducePullKernelPtr(DataType dt, int nranks);
+const void* reducePullCastKernelFor(DataType in, DataType out, int nranks);  // nullptr: unsupported pair
+const void* gatherPushCastKernelFor(DataType in, DataType out);
 // Flag-in-data exchange for small messages (no barrier): mode 0 = allgather (my block to
 // everyone), 1 = alltoall (block j of my input to rank j). `bytes` per block, uniform.
 void launchLLExchange(const CommArgs& a, const void* in, void* out, size_t bytes, int mode, const PeerPtrs& ll,

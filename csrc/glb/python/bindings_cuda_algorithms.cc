@@ -204,6 +204,33 @@ void registerCudaAlgorithms(py::module_& m) {
     reduce_scatter(pc, P(in), P(out), counts, static_cast<DataType>(dtype), static_cast<ReduceOp>(op), S(st), scale);
   }, py::arg("pc"), py::arg("input"), py::arg("output"), py::arg("counts"), py::arg("dtype"), py::arg("op") = 1,
      py::arg("stream") = 0, py::arg("scale") = 1.0);
+  // With a dtype conversion (f32 <-> f16 / bf16). Counts are ELEMENTS: input and output
+  // element sizes differ.
+  m.def("reduce_scatter_cast_reg", [](PeerContext& pc, const PeerBuffer& in, size_t off, uintptr_t out,
+                                      std::vector<size_t> counts, int dtype, int outDtype, int op, uintptr_t st,
+                                      double scale) {
+    py::gil_scoped_release nogil;
+    reduceScatterCast(pc, in, off, P(out), counts, static_cast<DataType>(dtype), static_cast<DataType>(outDtype),
+                      static_cast<ReduceOp>(op), S(st), scale);
+  }, py::arg("pc"), py::arg("input"), py::arg("offset"), py::arg("output"), py::arg("counts"), py::arg("dtype"),
+     py::arg("out_dtype"), py::arg("op") = 1, py::arg("stream") = 0, py::arg("scale") = 1.0);
+  m.def("reduce_scatter_cast", [](PeerContext& pc, uintptr_t in, uintptr_t out, std::vector<size_t> counts, int dtype,
+                                  int outDtype, int op, uintptr_t st, double scale) {
+    py::gil_scoped_release nogil;
+    reduceScatterCast(pc, P(in), P(out), counts, static_cast<DataType>(dtype), static_cast<DataType>(outDtype),
+                      static_cast<ReduceOp>(op), S(st), scale);
+  }, py::arg("pc"), py::arg("input"), py::arg("output"), py::arg("counts"), py::arg("dtype"), py::arg("out_dtype"),
+     py::arg("op") = 1, py::arg("stream") = 0, py::arg("scale") = 1.0);
+  m.def("allgatherv_cast_reg", [](PeerContext& pc, uintptr_t in, int dtype, const PeerBuffer& out, size_t off,
+                                  std::vector<size_t> counts, int outDtype, uintptr_t st) {
+    py::gil_scoped_release nogil;
+    allgathervCast(pc, P(in), static_cast<DataType>(dtype), out, off, counts, static_cast<DataType>(outDtype), S(st));
+  });
+  m.def("allgatherv_cast", [](PeerContext& pc, uintptr_t in, int dtype, uintptr_t out, std::vector<size_t> counts,
+                              int outDtype, uintptr_t st) {
+    py::gil_scoped_release nogil;
+    allgathervCast(pc, P(in), static_cast<DataType>(dtype), P(out), counts, static_cast<DataType>(outDtype), S(st));
+  });
   m.def("reduce_reg", [](PeerContext& pc, const PeerBuffer& in, size_t inOff, const PeerBuffer& out, size_t outOff,
                          size_t count, int dtype, int op, int root, uintptr_t st) {
     py::gil_scoped_release nogil;

@@ -45,6 +45,37 @@ def _algo(a) -> int:
     return ALGOS[a] if isinstance(a, str) else int(a)
 
 
+# (input, output) dtypes that reduce_scatter / allgather(v) convert inside the kernel
+CAST_PAIRS = frozenset({(DataType.FLOAT32, DataType.FLOAT16), (DataType.FLOAT32, DataType.BFLOAT16),
+                        (DataType.FLOAT16, DataType.FLOAT32), (DataType.BFLOAT16, DataType.FLOAT32)})
+
+
+def _cast_types(what: str, in_dtype, out_dtype) -> Tuple[DataType, DataType]:
+    """DataTypes of a converting call from torch dtypes ``in_dtype`` -> ``out_dtype`` (which
+    differ); TypeError for any pair outside ``CAST_PAIRS``. Same-dtype calls never come here: they
+    move raw bytes of any dtype, including those without a DataType (float8, complex, uint16...)."""
+    try:
+        pair = (_torch_dtype_to_glb(in_dtype), _torch_dtype_to_glb(out_dtype))
+    except KeyError:
+        pair = None
+    if pair not in CAST_PAIRS:
+        raise TypeError(f"{what}: cannot convert {in_dtype} to {out_dtype}; the supported conversions are "
+                        "FLOAT32 -> FLOAT16 / BFLOAT16 and FLOAT16 / BFLOAT16 -> FLOAT32")
+    return pair
+
+
+def _check_counts(what: str, counts: Sequence[int], size: int) -> List[int]:
+    counts = [int(c) for c in counts]
+    if len(counts) != size or any(c < 0 for c in counts):
+        raise ValueError(f"{what}: need {size} non-negative element counts, got {counts}")
+    return counts
+
+
+def _check_len(what: str, name: str, have: int, need: int) -> None:
+    if have < need:
+        raise ValueError(f"{what}: {name} holds {have} elements, the counts need {need}")
+
+
 def new_stream(device: Optional[int] = None, high_priority: bool = False):
     """A dedicated CUDA stream as a torch ExternalStream (never shared through torch's pool)."""
     import torch
@@ -255,13 +286,33 @@ class CudaContext:
         return tensor
 
     def allgather(self, output, input, stream=None):
+        """Every rank's ``input`` (same length on every rank), in rank order, in every ``output``.
+        ``output`` may have another dtype than ``input``: see ``allgatherv``."""
         return self.allgatherv(output, input, [input.numel()] * self.size, stream)
 
     def allgatherv(self, output, input, counts: Sequence[int], stream=None):
-        es = output.element_size()
-        sizes = [int(c) * es for c in counts]
+        """Rank r's ``input`` (``counts[r]`` elements) lands at element offset ``sum(counts[:r])`` of
+        every rank's ``output``.
+
+        With ``output.dtype != input.dtype`` (float32 -> float16 / bfloat16, or float16 / bfloat16 ->
+        float32) each rank's block is converted once inside the kernel: narrowing rounds to nearest
+        even (values beyond the float16 range become Inf), widening is exact. Only the output dtype
+        crosses NVLink. Raises ``ValueError`` when ``output`` or ``input`` is shorter than the counts
+        say and ``TypeError`` for any other dtype pair, before anything is launched."""
+        counts = _check_counts("allgatherv", counts, self.size)
+        _check_len("allgatherv", "output", output.numel(), sum(counts))
+        _check_len("allgatherv", "input", input.numel() if input is not None else 0, counts[self.rank])
         buf, off = self.lookup(output)
         iptr = input.data_ptr() if input is not None else 0
+        if input is not None and input.dtype != output.dtype:
+            idt, odt = _cast_types("allgatherv", input.dtype, output.dtype)
+            if buf is not None:
+                _cu.allgatherv_cast_reg(self.pc, iptr, int(idt), buf, off, counts, int(odt), _stream(stream))
+            else:
+                _cu.allgatherv_cast(self.pc, iptr, int(idt), output.data_ptr(), counts, int(odt), _stream(stream))
+            return output
+        es = output.element_size()
+        sizes = [c * es for c in counts]
         if buf is not None:
             _cu.allgatherv_reg(self.pc, iptr, buf, off, sizes, _stream(stream))
         else:
@@ -315,15 +366,36 @@ class CudaContext:
 
     def reduce_scatter(self, output, input, counts: Optional[Sequence[int]] = None, op: ReduceOp = ReduceOp.SUM,
                        stream=None, scale: float = 1.0):
+        """Rank r gets elements ``[sum(counts[:r]), +counts[r])`` of the reduction of every rank's
+        ``input`` in ``output`` (default counts: ``input`` split as evenly as possible).
+
+        With ``output.dtype != input.dtype`` (float32 -> float16 / bfloat16, or float16 / bfloat16 ->
+        float32) the kernel accumulates in float32, multiplies the accumulator by ``scale`` and rounds
+        once to the output dtype; the input dtype is what crosses NVLink. Raises ``ValueError`` when
+        ``output`` or ``input`` is shorter than the counts say and ``TypeError`` for any other dtype
+        pair, before anything is launched."""
+        cast = _cast_types("reduce_scatter", input.dtype, output.dtype) if output.dtype != input.dtype else None
         ptr, n, dt, _ = describe(input)
         if counts is None:
             base, rem = divmod(n, self.size)
             counts = [base + (1 if r < rem else 0) for r in range(self.size)]
+        counts = _check_counts("reduce_scatter", counts, self.size)
+        _check_len("reduce_scatter", "input", n, sum(counts))
+        _check_len("reduce_scatter", "output", output.numel(), counts[self.rank])
         buf, off = self.lookup(input)
+        if cast is not None:
+            odt = cast[1]
+            if buf is not None:
+                _cu.reduce_scatter_cast_reg(self.pc, buf, off, output.data_ptr(), counts, int(dt), int(odt), int(op),
+                                            _stream(stream), scale)
+            else:
+                _cu.reduce_scatter_cast(self.pc, ptr, output.data_ptr(), counts, int(dt), int(odt), int(op),
+                                        _stream(stream), scale)
+            return output
         if buf is not None:
-            _cu.reduce_scatter_reg(self.pc, buf, off, output.data_ptr(), list(counts), int(dt), int(op), _stream(stream), scale)
+            _cu.reduce_scatter_reg(self.pc, buf, off, output.data_ptr(), counts, int(dt), int(op), _stream(stream), scale)
         else:
-            _cu.reduce_scatter(self.pc, ptr, output.data_ptr(), list(counts), int(dt), int(op), _stream(stream), scale)
+            _cu.reduce_scatter(self.pc, ptr, output.data_ptr(), counts, int(dt), int(op), _stream(stream), scale)
         return output
 
     def reduce(self, output, input, root: int = 0, op: ReduceOp = ReduceOp.SUM, stream=None):

@@ -238,6 +238,9 @@ class ZeroShard(_Base):
         return start, counts[self.rank], counts
 
     def reduce_scatter_gradients(self, flat_grad, out_shard, average: bool = True):
+        """``out_shard`` may have another dtype than ``flat_grad`` (e.g. bf16 gradients into an fp32
+        shard): on CUDA the kernel converts (fp32 accumulation, 1/P on the accumulator, one
+        rounding); on the host the gradient is converted with torch first."""
         _, _, counts = self.shard_range(flat_grad.numel())
         if _is_cuda(flat_grad):
             fused = average and flat_grad.is_floating_point()
@@ -245,16 +248,23 @@ class ZeroShard(_Base):
             if average and not fused:
                 out_shard.div_(self.size)
         else:
+            if getattr(flat_grad, "dtype", None) != getattr(out_shard, "dtype", None):
+                flat_grad = flat_grad.to(out_shard.dtype)
             H.reduce_scatter(self.ctx, out_shard, flat_grad, counts)
             if average:
                 out_shard.div_(self.size) if hasattr(out_shard, "div_") else None
         return out_shard
 
     def allgather_parameters(self, flat_param, shard):
+        """``shard`` may have another dtype than ``flat_param`` (e.g. an fp32 master shard gathered
+        into bf16 parameters): on CUDA each shard is converted once inside the kernel; on the host it
+        is converted with torch first."""
         _, _, counts = self.shard_range(flat_param.numel())
         if _is_cuda(flat_param):
             self.cc.allgatherv(flat_param, shard, counts)
         else:
+            if getattr(flat_param, "dtype", None) != getattr(shard, "dtype", None):
+                shard = shard.to(flat_param.dtype)
             H.allgatherv(self.ctx, flat_param, counts, shard)
         return flat_param
 
@@ -270,9 +280,20 @@ class ZeroOptimizer(_Base):
 
         zo = ZeroOptimizer(ctx, cuda_ctx, model.parameters(), torch.optim.AdamW, lr=1e-3)
         loss.backward(); zo.step(); zo.zero_grad()
+
+    ``master_dtype`` (e.g. ``torch.float32`` for a bf16 / fp16 model) gives the optimizer master
+    weights of that dtype: the shard and its gradient are ``master_dtype``, initialised from the
+    upcast parameters, while the flat parameter and gradient buffers stay in the model dtype. On
+    CUDA ``step()`` is then still two collective launches: a reduce_scatter that converts the
+    gradients (fp32 accumulation, 1/P and one rounding inside the kernel) and an allgather that
+    rounds the updated master shard once into the model dtype. ``None`` keeps one dtype.
+    Exception: with a single rank both conversions run locally through the small-message (LL)
+    kernel, one launch per ``GLB_CUDA_LL_MAX``-sized piece (16 KB by default), which is far slower
+    than the same step without ``master_dtype`` for large models (see docs/cuda.md).
     """
 
-    def __init__(self, ctx, cuda_ctx, params: Iterable, optimizer_cls, average: bool = True, **optimizer_kwargs):
+    def __init__(self, ctx, cuda_ctx, params: Iterable, optimizer_cls, average: bool = True, master_dtype=None,
+                 **optimizer_kwargs):
         import torch
 
         super().__init__(ctx, cuda_ctx)
@@ -304,7 +325,14 @@ class ZeroOptimizer(_Base):
         cnt = self.counts[self.rank]
         # the shard the optimizer owns: its own tensors (the collectives' inputs / outputs must not
         # alias the flat buffers they gather into / scatter from)
-        self.shard = torch.nn.Parameter(self.flat_param[self.start:self.start + cnt].detach().clone())
+        # The padding above starts every shard on a 16-byte boundary of the model-dtype buffers, which
+        # keeps the converting collectives on their vector path as well.
+        src = self.flat_param[self.start:self.start + cnt].detach()
+        self.master_dtype = master_dtype
+        if master_dtype is None:
+            self.shard = torch.nn.Parameter(src.clone())
+        else:
+            self.shard = torch.nn.Parameter(src.to(master_dtype, copy=True))
         self.shard.grad = torch.zeros_like(self.shard)
         self.optimizer = optimizer_cls([self.shard], **optimizer_kwargs)
 
